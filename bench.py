@@ -4,6 +4,7 @@ at 384^2).
 
     python bench.py [--gpus N --steps K --warmup W]            # our arm (N>1: under torchrun)
     python bench.py --impl reference [...]                      # CPU arm: the unmodified reference module (oracle/_ref)
+    python bench.py [...] --dump-outputs DIR                    # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = one pass of the hot path (prompt_encoder + 16 ShapePropDecoders + injection layout,
 cod.py:1467-1505 minus the PVT blocks) over one batch of synthetic RGB-D input.  Workload =
@@ -53,7 +54,13 @@ def parse():
     ap.add_argument("--no-highres", action="store_true")
     ap.add_argument("--no-backbone", action="store_true")
     ap.add_argument("--train-batch", type=int, default=16, help="images per GPU per training step (configs[2])")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the last timed step returned (rank 0) as DIR/<name>.npy, float32; tensors above "
+                         "the per-tensor share of 48 MiB are reduced to a fixed, seeded sample of their elements")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -635,6 +642,29 @@ def full_model_train_bench(dev, world, rank, args, common, sharding, steps=5, wa
             "allreduce_exposed_ms": exposed}
 
 
+DUMP_BYTES = 48 << 20
+
+
+def dump_outputs(outdir: str, e1, toks) -> None:
+    """Write embedding1 and the prompt tokens of one hot-path step as `<name>.npy` (names of
+    `common.flatten_outputs`), float32, so that two builds can be compared output for output.  A tensor
+    with more elements than its share of DUMP_BYTES keeps at most that many, at distinct flat indices drawn
+    from a generator seeded by the tensor's name: the same arguments select the same elements in every run."""
+    import zlib
+    import numpy as np
+    import common
+    named = {k: v for k, v in common.flatten_outputs(e1, None, toks).items() if v is not None}
+    cap = DUMP_BYTES // (4 * len(named))
+    os.makedirs(outdir, exist_ok=True)
+    for name, t in named.items():
+        flat = t.detach().reshape(-1)
+        if flat.numel() > cap:
+            g = torch.Generator("cpu").manual_seed(zlib.crc32(name.encode()))
+            idx = torch.randint(flat.numel(), (cap,), generator=g).unique()
+            flat = flat[idx.to(flat.device)]
+        np.save(os.path.join(outdir, name + ".npy"), flat.float().cpu().numpy())
+
+
 def capi_launches() -> int:
     from dgtd_b200.twig.ops import capi
     return capi.launch_count()
@@ -847,12 +877,16 @@ def run_ours(args):
     n0 = capi.launch_count()
     with ClockSampler(local) as clocks:
         for a, b in ev:
+            outs = None                         # the previous step's outputs are freed before the next step runs
             flush.zero_()                       # L2 flush between timed iterations (not timed)
             a.record()
-            step(image, depth)
+            outs = step(image, depth)
             b.record()
         barrier()
     launches = capi.launch_count() - n0
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, outs[0], outs[2])
+    outs = None
     from dgtd_b200.twig import sharding
     t_dev = sum(a.elapsed_time(b) for a, b in ev) / 1e3
     t_max = sharding.max_over_ranks(t_dev, dev)                     # device time, max over ranks
@@ -865,7 +899,7 @@ def run_ours(args):
     res_h = [torch.empty(B, (S // 32) ** 2, 512, dtype=torch.float32).pin_memory() for _ in range(2)]   # last-stage prompt tokens
     pipe = HostPipeline(enc, dec, precision=args.precision, want_embedding3=False, device=dev)
     select = lambda e1, e3, toks: toks[3][2].float()
-    e2e_steps = max(3, args.steps)   # the same K as the device-timed loop; the un-overlapped first copy (pipeline fill) is inside
+    e2e_steps = args.steps   # the same K as the device-timed loop; the un-overlapped first copy (pipeline fill) is inside
     for _ in pipe.run([(image_h, depth_h)] * 2, select, res_h):   # warm the pipeline's buffers
         pass
     barrier()
