@@ -253,7 +253,5 @@ PFN_tmapEncodeTiled get_tmap_encoder();  // nullptr on failure (error string set
 int make_tmap(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int rank,
               const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
               CUtensorMapSwizzle swz);
-int make_tmap_promo(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int rank, const uint64_t* dims,
-                    const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapL2promotion promo);
 
 }  // namespace dgtd

@@ -272,21 +272,12 @@ int d3_make_tmap(CUtensorMap* tm, const void* x, int B, int h, int w, int C) {
   return 0;
 }
 
-bool d3_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("DGTD_DW3_TMA");
-    on = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
-}
-
 }  // namespace
 
 // Returns 1 when the shape is not handled here (the caller falls through to the register-window kernel).
 int dwconv3_gelu_tma(const void* x, const float* wT, const float* bias, void* out, int B, int h, int w, int C,
                      cudaStream_t s) {
-  if (!d3_enabled() || C % 64 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(out) & 15)) return 1;
+  if (C % 64 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(out) & 15)) return 1;
   CUtensorMap tm;
   int rc = d3_make_tmap(&tm, x, B, h, w, C);
   if (rc) return rc;
@@ -310,7 +301,7 @@ int64_t dwconv3_gelu_bwd_tma_ws_floats() { return (int64_t)512 * 640; }   // per
 // Returns 1 when the shape is not handled here.
 int dwconv3_gelu_bwd_tma(const void* x, const float* wT, const float* bias, const float* g, float* du, float* dwT,
                          float* dbias, float* ws, int B, int h, int w, int C, cudaStream_t s) {
-  if (!d3_enabled() || !ws || C % 64 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(g) & 15) ||
+  if (!ws || C % 64 || (reinterpret_cast<uintptr_t>(x) & 15) || (reinterpret_cast<uintptr_t>(g) & 15) ||
       (reinterpret_cast<uintptr_t>(du) & 15))
     return 1;
   CUtensorMap tm;

@@ -320,14 +320,6 @@ namespace dgtd {
 int64_t attention_bwd_tc_ws_floats(int B, int N, int Nk, int heads);   // attn_bwd_tc.cu
 int attention_bwd_tc(const void* q, const void* kv, const void* o, const float* dout, float* dq, float* dkv, float* ws, int B,
                      int N, int Nk, int heads, float scale, cudaStream_t s);
-static bool attention_bwd_tc_enabled() {
-  static int on = -1;
-  if (on < 0) {
-    const char* e = getenv("DGTD_ATTN_BWD_TC");
-    on = (e && e[0] == '0') ? 0 : 1;
-  }
-  return on == 1;
-}
 int64_t dwconv3_gelu_bwd_tma_ws_floats();   // dwconv3_tma.cu
 int dwconv3_gelu_bwd_tma(const void* x, const float* wT, const float* bias, const float* g, float* du, float* dwT,
                          float* dbias, float* ws, int B, int h, int w, int C, cudaStream_t s);
@@ -346,7 +338,7 @@ int dgtd_attention_bwd(const void* q, const void* kv, const void* out, const flo
   DGTD_CHECK_ARG(dtype == DGTD_F32 || dtype == DGTD_BF16, "attention_bwd: bad dtype %d", dtype);
   const int C = heads * AB_D;
   cudaStream_t s = (cudaStream_t)stream;
-  if (dtype == DGTD_BF16 && attention_bwd_tc_enabled()) {   // mma.sync path, no atomics (attn_bwd_tc.cu)
+  if (dtype == DGTD_BF16) {   // mma.sync path, no atomics (attn_bwd_tc.cu)
     const int rc = attention_bwd_tc(q, kv, out, dout, dq, dkv, ws, B, N, Nk, heads, scale, s);
     if (rc) return rc;
     DGTD_LAUNCH_CHECK("attention_bwd(tc)");
@@ -358,22 +350,12 @@ int dgtd_attention_bwd(const void* q, const void* kv, const void* out, const flo
   DGTD_CHECK_ARG(e == cudaSuccess, "attention_bwd: memset failed: %s", cudaGetErrorString(e));
   const size_t smem = (size_t)(6 * AB_T * AB_P + 2 * AB_T) * sizeof(float);
   dim3 gs(cdiv(N, AS_QB), heads, B), gb(cdiv(N, AB_QCH), heads, B);
-  if (dtype == DGTD_BF16) {
-    e = cudaFuncSetAttribute(attention_bwd_kernel<__nv_bfloat16>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    DGTD_CHECK_ARG(e == cudaSuccess, "attention_bwd: cannot opt in to %zu B smem", smem);
-    attention_stats_kernel<<<gs, 256, 0, s>>>((const __nv_bfloat16*)q, (const __nv_bfloat16*)kv, (const __nv_bfloat16*)out,
-                                               dout, lse, dsum, N, Nk, C, scale);
-    DGTD_LAUNCH_CHECK("attention_stats");
-    attention_bwd_kernel<<<gb, 256, smem, s>>>((const __nv_bfloat16*)q, (const __nv_bfloat16*)kv, dout, lse, dsum, dq, dkv,
-                                                N, Nk, C, scale);
-  } else {
-    e = cudaFuncSetAttribute(attention_bwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-    DGTD_CHECK_ARG(e == cudaSuccess, "attention_bwd: cannot opt in to %zu B smem", smem);
-    attention_stats_kernel<<<gs, 256, 0, s>>>((const float*)q, (const float*)kv, (const float*)out, dout, lse, dsum, N, Nk,
-                                               C, scale);
-    DGTD_LAUNCH_CHECK("attention_stats");
-    attention_bwd_kernel<<<gb, 256, smem, s>>>((const float*)q, (const float*)kv, dout, lse, dsum, dq, dkv, N, Nk, C, scale);
-  }
+  e = cudaFuncSetAttribute(attention_bwd_kernel<float>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+  DGTD_CHECK_ARG(e == cudaSuccess, "attention_bwd: cannot opt in to %zu B smem", smem);
+  attention_stats_kernel<<<gs, 256, 0, s>>>((const float*)q, (const float*)kv, (const float*)out, dout, lse, dsum, N, Nk,
+                                             C, scale);
+  DGTD_LAUNCH_CHECK("attention_stats");
+  attention_bwd_kernel<<<gb, 256, smem, s>>>((const float*)q, (const float*)kv, dout, lse, dsum, dq, dkv, N, Nk, C, scale);
   DGTD_LAUNCH_CHECK("attention_bwd");
   return 0;
 }

@@ -7,7 +7,6 @@
 // out-of-bounds = zero padding) into a 64B-swizzled K-major smem tile that tcgen05.mma consumes.
 // Groups (the 16 decoders of the path) are a grid dimension: group g reads channel slice
 // [32g, 32g+32) of x, weight rows [g*w_group_rows, ...) and writes out + g*out_group_stride.
-#include <stdlib.h>
 #include "blackwell.cuh"
 #include "common.cuh"
 
@@ -725,26 +724,14 @@ static int conv_halo_launch(const void* x, int B, int h, int wd, int ldx, int64_
     uint64_t dims[4] = {(uint64_t)ldx, (uint64_t)wd, (uint64_t)h, (uint64_t)B};
     uint64_t str[3] = {(uint64_t)ldx * 2, (uint64_t)wd * ldx * 2, (uint64_t)h * wd * ldx * 2};
     uint32_t box[4] = {32, HALO_PW, HALO_PH, 1};
-    // 64-byte channel slices of pixel rows that interleave all groups (ldx * 2 bytes per pixel): how far L2 widens each
-    // request decides how much of the neighbouring groups' slices is dragged in (and evicted again before their CTAs
-    // arrive).  DGTD_HALO_L2PROMO = 0 / 64 / 128 / 256 for A/B runs.
-    static int promo_sel = -1;
-    if (promo_sel < 0) {
-      const char* e = getenv("DGTD_HALO_L2PROMO");
-      promo_sel = e ? atoi(e) : 256;
-    }
-    const CUtensorMapL2promotion promo = promo_sel == 0     ? CU_TENSOR_MAP_L2_PROMOTION_NONE
-                                         : promo_sel == 64  ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                                         : promo_sel == 128 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B
-                                                            : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
     int rc;
     if (p.x5d) {   // group-major: every group is a dense (B, h, w, 32) tensor, xgs elements apart
       uint64_t dims5[5] = {32, (uint64_t)wd, (uint64_t)h, (uint64_t)B, (uint64_t)p.groups};
       uint64_t str5[4] = {(uint64_t)ldx * 2, (uint64_t)wd * ldx * 2, (uint64_t)h * wd * ldx * 2, (uint64_t)xgs * 2};
       uint32_t box5[5] = {32, HALO_PW, HALO_PH, 1, 1};
-      rc = make_tmap_promo(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, dims5, str5, box5, CU_TENSOR_MAP_SWIZZLE_64B, promo);
+      rc = make_tmap(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 5, dims5, str5, box5, CU_TENSOR_MAP_SWIZZLE_64B);
     } else {
-      rc = make_tmap_promo(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B, promo);
+      rc = make_tmap(&tmX, x, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, dims, str, box, CU_TENSOR_MAP_SWIZZLE_64B);
     }
     if (rc) return rc;
   }
@@ -820,12 +807,7 @@ static int conv_launch(const CUtensorMap& tmX, const __nv_bfloat16* w, int Ktot,
     using Rw = ConvRwCfg<BN>;
     const int keys = p.groups * p.tiles_n;
     const int64_t per_key = (int64_t)p.B * p.tiles_x * p.tiles_y;
-    static int use_rw = -1;
-    if (use_rw < 0) {
-      const char* e = getenv("DGTD_CONV_RESW");
-      use_rw = e ? atoi(e) : 1;
-    }
-    if (use_rw && BN >= 64 && keys <= sm_count() && p.ks * p.ks <= Rw::MAX_TAPS && per_key < (1ll << 31)) {
+    if (BN >= 64 && keys <= sm_count() && p.ks * p.ks <= Rw::MAX_TAPS && per_key < (1ll << 31)) {
       auto kern_rw = tc_conv_resw_kernel<BN, ACT, OT>;
       static bool configured_rw = false;
       if (!configured_rw) {
@@ -886,12 +868,12 @@ int tc_conv_nhwc(const void* x, const void* w, const float* bias, void* out, int
     set_error("conv_nhwc(bf16): x_group_stride must be a multiple of 8 elements");
     return -1;
   }
-  const bool halo_ok = ks == 3 && stride == 1 && off == -1 && oh == h && ow == wd && !getenv("DGTD_CONV_NO_HALO");
+  const bool halo_ok = ks == 3 && stride == 1 && off == -1 && oh == h && ow == wd;
   if (p.out_split && !(halo_ok && dtype_out == DGTD_BF16 && Cout % 32 == 0)) {
     set_error("conv_nhwc(bf16): the chunk-scattered output needs the 3x3 stride-1 conv, bf16 output and Cout %% 32 == 0");
     return -1;
   }
-  if (ks == 3 && stride == 1 && off == -1 && oh == h && ow == wd && !getenv("DGTD_CONV_NO_HALO")) {
+  if (halo_ok) {
     const int Wrows = groups * w_group_rows;
     const __nv_bfloat16* wp = (const __nv_bfloat16*)w;
     if (dtype_out == DGTD_BF16) {

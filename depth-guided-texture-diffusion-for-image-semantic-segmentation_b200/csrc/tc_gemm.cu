@@ -32,17 +32,9 @@ PFN_tmapEncodeTiled get_tmap_encoder() {
   return fn;
 }
 
-int make_tmap_promo(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int rank, const uint64_t* dims,
-                    const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapL2promotion promo);
-
 int make_tmap(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int rank,
               const uint64_t* dims, const uint64_t* strides_bytes, const uint32_t* box,
               CUtensorMapSwizzle swz) {
-  return make_tmap_promo(out, base, dt, rank, dims, strides_bytes, box, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B);
-}
-
-int make_tmap_promo(CUtensorMap* out, const void* base, CUtensorMapDataType dt, int rank, const uint64_t* dims,
-                    const uint64_t* strides_bytes, const uint32_t* box, CUtensorMapSwizzle swz, CUtensorMapL2promotion promo) {
   PFN_tmapEncodeTiled enc = get_tmap_encoder();
   if (!enc) return -3;
   cuuint64_t gd[5], gs[5];
@@ -54,7 +46,7 @@ int make_tmap_promo(CUtensorMap* out, const void* base, CUtensorMapDataType dt, 
     if (i > 0) gs[i - 1] = strides_bytes[i - 1];
   }
   CUresult r = enc(out, dt, (cuuint32_t)rank, const_cast<void*>(base), gd, gs, bx, es,
-                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, promo,
+                   CU_TENSOR_MAP_INTERLEAVE_NONE, swz, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) {
     set_error("cuTensorMapEncodeTiled failed (CUresult %d) rank=%d dims=[%llu,%llu] box=[%u,%u]", (int)r,

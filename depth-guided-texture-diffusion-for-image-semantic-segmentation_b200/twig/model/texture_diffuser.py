@@ -36,7 +36,6 @@ __all__ = [
 # centres in fp32 AFTER the bf16 rounding of the un-normalised conv output, i.e. it loses accuracy when a pixel's
 # channel mean dwarfs its channel spread (|mean| >> std); DGTD_LN_FOLD=0 keeps the two-pass form.
 LN_FOLD = os.environ.get("DGTD_LN_FOLD", "1") != "0"
-MLP_FUSED = os.environ.get("DGTD_MLP_FUSED", "1") != "0"   # A/B switch of the fused stage-0 MLP kernel
 
 PVT_EMBED_DIMS = (64, 128, 320, 512)  # pvt_v2_b2, cod.py:1785
 PVT_DEPTHS = (3, 4, 6, 3)             # cod.py:1786
@@ -238,7 +237,7 @@ class convnext_Block(nn.Module):
                         (w1f @ self.norm.bias.detach().float() + self.pwconv1.bias.detach().float()).contiguous())
             wq, col_s, cbias = pk.get("w1.lnfold", [self.pwconv1.weight, self.pwconv1.bias, self.norm.weight, self.norm.bias], fold)
             y, stats = OP.dwconv7_stats_tma(x, dw_wT, self.dwconv.bias.detach(), self.norm.eps)
-            if MLP_FUSED and keep is None and C in OP.MLP_FUSED_C and (B * h * w) % 128 == 0:
+            if keep is None and C in OP.MLP_FUSED_C and (B * h * w) % 128 == 0:
                 # stage 0: both pointwise GEMMs in one kernel, the 4C hidden tensor never reaches HBM
                 OP.convnext_mlp_fused_(y.view(-1, C), stats, wq, col_s, cbias, w2, self.pwconv2.bias.detach(), gamma, x)
                 return x
@@ -326,7 +325,7 @@ class ShapePropEncoder(nn.Module):
             w0b = pk.get("stem.bf16", [st_conv.weight], lambda: w0.to(torch.bfloat16))
             B, _, H, W = image.shape
             patches = OP.stem_patches(image, grid, BF16)
-            if _STEM_LN_FUSED and self.dims[0] == 128 and patches.shape[0] >= 256:
+            if self.dims[0] == 128 and patches.shape[0] >= 256:
                 # the row LayerNorm in the GEMM's epilogue: the fp32 map is written once instead of written, read and rewritten
                 x = OP.linear_ln(patches, w0b, st_conv.bias.detach().float(), st_ln.weight.detach().float(),
                                  st_ln.bias.detach().float(), st_ln.eps).view(B, H // 4, W // 4, self.dims[0])
@@ -360,24 +359,18 @@ class ShapePropEncoder(nn.Module):
             conv = self.convs[i]
             # fusion conv folded into the head projection (both 1x1, and a 1x1 conv commutes with the bilinear
             # up-sample): z_i = x_i (Wf_i Wh_i)^T + Wf_i bh_i, so the 96 -> 24 product at full resolution is gone
-            wl = pk.get(f"headf{i}.{mode}", [conv.weight, fw],
-                        lambda conv=conv, i=i: _as(fw.detach().reshape(L, 4 * L)[:, i * L:(i + 1) * L].float()
-                                                   @ conv.weight.detach().reshape(L, -1).float(), mode))
+            wl = pk.get(f"headf{i}", [conv.weight, fw],
+                        lambda conv=conv, i=i: (fw.detach().reshape(L, 4 * L)[:, i * L:(i + 1) * L].float()
+                                                @ conv.weight.detach().reshape(L, -1).float()).contiguous())
             bl = pk.get(f"headfb{i}", [conv.bias, fw],
                         lambda conv=conv, i=i: (fw.detach().reshape(L, 4 * L)[:, i * L:(i + 1) * L].float()
                                                 @ conv.bias.detach().float()).contiguous())
             a = o.view(-1, o.shape[-1])
-            if mode == BF16 and _HEAD_TF32 and L % 8 == 0 and L <= 64:
+            if mode == BF16 and L % 8 == 0 and L <= 64:
                 # tcgen05 projection (N = 24) straight from the fp32 stage output: TF32 products, no bf16 copy
-                w32 = pk.get(f"headf{i}.tf32", [conv.weight, fw],
-                             lambda conv=conv, i=i: (fw.detach().reshape(L, 4 * L)[:, i * L:(i + 1) * L].float()
-                                                     @ conv.weight.detach().reshape(L, -1).float()).contiguous())
-                levels.append(OP.linear_tf32(a, w32, bl))
-                hw.append((o.shape[1], o.shape[2]))
-                continue
-            if mode == BF16:       # tcgen05 projection (N=24): cast the fp32 stage output once
-                a = OP.cast(a, torch.bfloat16)
-            levels.append(OP.linear(a, wl, bl, out_dtype=F32))
+                levels.append(OP.linear_tf32(a, wl, bl))
+            else:
+                levels.append(OP.linear(a, wl, bl, out_dtype=F32))
             hw.append((o.shape[1], o.shape[2]))
         return OP.fusion_sum(levels, hw, self.fusion_conv.bias.detach(), B, want_nhwc=True, want_nchw=want_nchw,
                              pad_to=pad_to)
@@ -490,17 +483,9 @@ def _decoder_front(decoders: Sequence[ShapePropDecoder], emb: torch.Tensor) -> t
     return h2
 
 
-# stem of the bf16 mode: LayerNorm fused in the K = 48 GEMM's epilogue (default) or as a separate in-place pass (DGTD_STEM_LN=0)
-_STEM_LN_FUSED = os.environ.get("DGTD_STEM_LN", "1") != "0"
-# head projections of the bf16 mode on kind::tf32 from the fp32 stage outputs (default) or on bf16 copies (DGTD_HEAD_TF32=0)
-_HEAD_TF32 = os.environ.get("DGTD_HEAD_TF32", "1") != "0"
-# hidden maps of the bf16 decoder bank: group-major (default) or interleaved channel slices (DGTD_DEC_GROUP_MAJOR=0, A/B)
-_GROUP_MAJOR = os.environ.get("DGTD_DEC_GROUP_MAJOR", "1") != "0"
-
-
 def _decoder_front_bf16(decoders: Sequence[ShapePropDecoder], emb_pad: torch.Tensor) -> torch.Tensor:
     """tcgen05 path: emb_pad NHWC (B,h,w,32) bf16 (24 latent channels + zero pad) ->
-    (B,h,w,32*D) bf16; decoder d owns channels [32d, 32d+24), the pad channels stay zero."""
+    (D,B,h,w,32) bf16; decoder d owns h2[d], channels [0, 24), the pad channels stay zero."""
     B, h, w, _ = emb_pad.shape
     D = len(decoders)
     L = decoders[0].decoder[0].in_channels
@@ -514,14 +499,8 @@ def _decoder_front_bf16(decoders: Sequence[ShapePropDecoder], emb_pad: torch.Ten
                 lambda: torch.cat([_pad_taps_bf16(_pack_conv3(d.decoder[2].weight), L, 32) for d in decoders], 0).contiguous())
     b2 = pk.get(key + ".b2", [d.decoder[2].bias for d in decoders],
                 lambda: torch.cat([_pad_rows(d.decoder[2].bias, 32) for d in decoders]).contiguous())
-    if not _GROUP_MAJOR:   # interleaved slices: decoder d owns channels [32d, 32d+32) of every pixel row
-        h1 = torch.empty(B, h, w, 32 * D, device=emb_pad.device, dtype=torch.bfloat16)
-        OP.conv_nhwc_grouped(emb_pad, w1, b1, 32, (h, w), 3, 1, -1, ACT_RELU, h1, 32 * D, 32 * D, 1, 0, 32 * D, 0)
-        h2 = torch.empty_like(h1)
-        OP.conv_nhwc_grouped(h1, w2, b2, 32, (h, w), 3, 1, -1, ACT_RELU, h2, 32, 32 * D, D, 32, 32, 32)
-        return h2
     # group-major: every decoder's hidden map is its own dense (B,h,w,32) tensor, so each halo box is made of whole
-    # 64-byte pixel rows that no other group's CTA shares (the interleaved form read 2.5x its input from DRAM)
+    # 64-byte pixel rows that no other group's CTA shares (interleaved channel slices read 2.5x their input from DRAM)
     gs = B * h * w * 32
     h1 = torch.empty(D, B, h, w, 32, device=emb_pad.device, dtype=torch.bfloat16)
     OP.conv_nhwc_grouped(emb_pad, w1, b1, 32, (h, w), 3, 1, -1, ACT_RELU, h1, 32 * D, 32, 1, 0, 32 * D, gs)
@@ -532,8 +511,9 @@ def _decoder_front_bf16(decoders: Sequence[ShapePropDecoder], emb_pad: torch.Ten
 
 def _decode_tokens_bf16(decoders: Sequence[ShapePropDecoder], h2: torch.Tensor, index0: int,
                         src_hw: Tuple[int, int], grid: Tuple[int, int]) -> List[torch.Tensor]:
-    """All decoders of one PVT stage in ONE grouped tcgen05 launch, output (D_s, B, H_s*W_s, E_s) bf16."""
-    B = h2.shape[-4]
+    """All decoders of one PVT stage in ONE grouped tcgen05 launch, output (D_s, B, H_s*W_s, E_s) bf16.
+    h2: the group-major hidden maps (D_all, B, h, w, 32) of ``_decoder_front_bf16``."""
+    B = h2.shape[1]
     D = len(decoders)
     E = decoders[0].decoder[4].out_channels
     L = decoders[0].decoder[4].in_channels
@@ -553,13 +533,8 @@ def _decode_tokens_bf16(decoders: Sequence[ShapePropDecoder], h2: torch.Tensor, 
     b3 = pk.get(key + ".b", [d.decoder[4].bias for d in decoders],
                 lambda: torch.cat([d.decoder[4].bias.detach().float() for d in decoders]).contiguous())
     out = torch.empty(D, B, grid[0] * grid[1], E, device=h2.device, dtype=torch.bfloat16)
-    if h2.dim() == 5:      # group-major hidden maps (D_all, B, h, w, 32)
-        OP.conv_nhwc_grouped(h2[index0], w3, b3, 32, grid, ks, stride, off, ACT_NONE, out, E, E, D, h2.stride(0), E,
-                             B * grid[0] * grid[1] * E)
-    else:
-        src = h2[..., index0 * 32:]
-        OP.conv_nhwc_grouped(src, w3, b3, 32, grid, ks, stride, off, ACT_NONE, out, E, E, D, 32, E,
-                             B * grid[0] * grid[1] * E)
+    OP.conv_nhwc_grouped(h2[index0], w3, b3, 32, grid, ks, stride, off, ACT_NONE, out, E, E, D, h2.stride(0), E,
+                         B * grid[0] * grid[1] * E)
     return [out[i] for i in range(D)]
 
 

@@ -29,7 +29,6 @@ SIGNATURES = {
     "dgtd_surface_normals_fwd": [_P, _P, _I, _I, _I, _P],
     "dgtd_lowpass_projector": [_P, _P, _I, _I, _P],
     "dgtd_fft_highpass_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
-    "dgtd_fft_highpass_tc_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
     "dgtd_fft_highpass_tc3_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
     "dgtd_diffusion_front_fwd": [_P] * 11 + [_I] * 6 + [_P],
     "dgtd_message_passing_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],

@@ -8,7 +8,6 @@ on the CPU or through ATen kernels.
 """
 from __future__ import annotations
 
-import os
 from typing import List, Optional, Sequence, Tuple
 
 import torch
@@ -104,10 +103,6 @@ class HighpassPlan:
         return plan
 
 
-# tcgen05 high-pass: one K-concatenated GEMM per product (default) or three accumulating GEMMs (DGTD_FFT_KCAT=0, A/B)
-_FFT_KCAT = os.environ.get("DGTD_FFT_KCAT", "1") != "0"
-
-
 def _split_bf16(t: torch.Tensor):
     hi = t.to(torch.bfloat16)
     return hi.contiguous(), (t - hi.float()).to(torch.bfloat16).contiguous()
@@ -120,7 +115,7 @@ def fft_highpass(x: torch.Tensor, rate: float = 0.3, tensor_cores: bool = False)
     assert x.dtype == torch.float32 and x.dim() == 4
     B, C, H, W = x.shape
     plan = HighpassPlan.get(H, W, rate, x.device)
-    if tensor_cores and H % 8 == 0 and W % 8 == 0 and _FFT_KCAT:
+    if tensor_cores and H % 8 == 0 and W % 8 == 0:
         # each split product as one K-concatenated GEMM: [x_hi | x_lo | x_hi] . [P_hi | P_hi | P_lo]^T
         if not hasattr(plan, "tc3"):
             def cat(t):
@@ -136,20 +131,6 @@ def fft_highpass(x: torch.Tensor, rate: float = 0.3, tensor_cores: bool = False)
         out = torch.empty_like(x)
         call("dgtd_fft_highpass_tc3_fwd", ptr(x), ptr(ph_cat), ptr(pw_cat), ptr(plan.sc_h), ptr(plan.sc_w), ptr(ws_a),
              ptr(ws_f), ptr(coef), ptr(out), B * C, H, W, stream())
-        return out
-    if tensor_cores and H % 8 == 0 and W % 8 == 0:
-        if not hasattr(plan, "tc"):
-            ph, pw = _split_bf16(plan.Ph), (_split_bf16(plan.Pw) if plan.Pw is not plan.Ph else None)
-            plan.tc = (ph, pw or ph, torch.zeros(max(H, W), device=x.device, dtype=torch.float32))
-        (ph_hi, ph_lo), (pw_hi, pw_lo), zeros = plan.tc
-        n = x.numel()
-        ws_hi = torch.empty(n, device=x.device, dtype=torch.bfloat16)
-        ws_lo = torch.empty(n, device=x.device, dtype=torch.bfloat16)
-        ws_f = torch.empty(n, device=x.device, dtype=torch.float32)
-        coef = torch.empty(B * C * 4, device=x.device, dtype=torch.float32)
-        out = torch.empty_like(x)
-        call("dgtd_fft_highpass_tc_fwd", ptr(x), ptr(ph_hi), ptr(ph_lo), ptr(pw_hi), ptr(pw_lo), ptr(plan.sc_h),
-             ptr(plan.sc_w), ptr(zeros), ptr(ws_hi), ptr(ws_lo), ptr(ws_f), ptr(coef), ptr(out), B * C, H, W, stream())
         return out
     tmp = torch.empty_like(x)
     coef = torch.empty(B * C * 4, device=x.device, dtype=torch.float32)

@@ -61,15 +61,9 @@ int dgtd_fft_highpass_fwd(const float* x, const float* Ph, const float* Pw, cons
                           const float* sc_w, float* tmp, float* coef, float* out, int planes,
                           int H, int W, dgtd_stream_t stream);
 /* Same operator with the two projector products on the tcgen05 GEMMs (bf16 mode of the path), fp32-accurate
- * through a two-term bf16 split of both operands (x_hi A_hi + x_hi A_lo + x_lo A_hi, fp32 accumulation).
- * P*_hi / P*_lo: bf16 split of the projectors; zeros: max(H,W) fp32 zeros; ws_hi / ws_lo: planes*H*W bf16,
- * ws_f32: planes*H*W fp32.  H, W multiples of 8. */
-int dgtd_fft_highpass_tc_fwd(const float* x, const void* Ph_hi, const void* Ph_lo, const void* Pw_hi, const void* Pw_lo,
-                             const float* sc_h, const float* sc_w, const float* zeros, void* ws_hi, void* ws_lo,
-                             float* ws_f32, float* coef, float* out, int planes, int H, int W, dgtd_stream_t stream);
-
-/* Same operator, each split product as ONE K-concatenated tcgen05 GEMM: [x_hi | x_lo | x_hi] . [A_hi | A_hi | A_lo]^T
- * (one fp32 accumulation in TMEM, no accumulator round trips through HBM).  Ph_cat / Pw_cat: [P_hi | P_hi | P_lo]
+ * through a two-term bf16 split of both operands (x_hi A_hi + x_hi A_lo + x_lo A_hi).  Each split product is ONE
+ * K-concatenated GEMM: [x_hi | x_lo | x_hi] . [A_hi | A_hi | A_lo]^T (one fp32 accumulation in TMEM, no accumulator
+ * round trips through HBM).  Ph_cat / Pw_cat: [P_hi | P_hi | P_lo]
  * per row (H x 3H, W x 3W bf16); ws_a: planes*H*W*3 bf16; ws_f32: planes*H*W fp32.  H, W multiples of 8. */
 int dgtd_fft_highpass_tc3_fwd(const float* x, const void* Ph_cat, const void* Pw_cat, const float* sc_h, const float* sc_w,
                               void* ws_a, float* ws_f32, float* coef, float* out, int planes, int H, int W,

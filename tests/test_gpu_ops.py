@@ -579,13 +579,11 @@ def test_fft_highpass_properties_at_full_size(OP):
     assert float((y[:, 2] - x[:, 2].abs()).abs().max()) < 1e-4
 
 
-@pytest.mark.parametrize("kcat", [True, False])
 @pytest.mark.parametrize("B,H,W", [(2, 384, 384), (1, 96, 160), (3, 352, 352)])
-def test_fft_highpass_tensor_core_variant_is_fp32_accurate(OP, B, H, W, kcat, monkeypatch):
-    """Projector products on tcgen05 with the two-term bf16 split: within 2e-5 of the float64 oracle (relative to
-    max|ref|), i.e. the same bar as the exact CUDA-core variant up to the split's 2^-16 terms.  kcat: each product
-    as one K-concatenated GEMM (the default) or as three accumulating GEMMs."""
-    monkeypatch.setattr(OP, "_FFT_KCAT", kcat)
+def test_fft_highpass_tensor_core_variant_is_fp32_accurate(OP, B, H, W):
+    """Projector products on tcgen05 with the two-term bf16 split, each product as one K-concatenated GEMM: within
+    2e-5 of the float64 oracle (relative to max|ref|), i.e. the same bar as the exact CUDA-core variant up to the
+    split's 2^-16 terms."""
     g = torch.Generator().manual_seed(H + W)
     x = torch.randn(B, 3, H, W, generator=g)
     ref = O.fft_highpass(x.double(), 0.3)

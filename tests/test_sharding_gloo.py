@@ -93,7 +93,10 @@ def _bucket_worker(rank, world, port, q):
     bk.calibrate()
     step()
     order = list(bk.launch_order)
-    q.put((rank, local, fg.clone(), [(b["lo"], b["hi"], b["need"]) for b in bk.buckets], order, offs, total))
+    # numpy arrays travel by value; a tensor would be shared by file descriptor from this process, which exits after
+    # the barrier below -- possibly before the parent has fetched it
+    q.put((rank, local.numpy(), fg.numpy().copy(), [(b["lo"], b["hi"], b["need"]) for b in bk.buckets], order, offs,
+           total))
     dist.barrier()
     dist.destroy_process_group()
 
@@ -111,6 +114,7 @@ def test_bucketed_gradient_allreduce_two_ranks():
         p.join(timeout=60)
         assert p.exitcode == 0
     (_, l0, g0, b0, o0, offs, total), (_, l1, g1, b1, o1, _, _) = res
+    l0, g0, l1, g1 = (torch.from_numpy(a) for a in (l0, g0, l1, g1))
     assert b0 == b1 and len(b0) >= 3
     # buckets tile the flat buffer from its END (reverse registration order = the order backward fills it)
     assert b0[0][1] == total and b0[-1][0] == 0 and all(a[0] == b[1] for a, b in zip(b0, b0[1:]))
