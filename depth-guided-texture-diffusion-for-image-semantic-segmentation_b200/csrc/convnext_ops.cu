@@ -268,68 +268,8 @@ dwconv7_ln_kernel(const float* __restrict__ x, const float* __restrict__ dw_w,
 }
 
 // ------------------------------------------------------------------------------------ a9 head tail
-// per output pixel: bilinear gather of the 4 projected levels (C ch each) -> 4C vector ->
-// 1x1 conv (C x 4C) + bias.  CTA = 32 pixels, 128 threads.
-template <int C>
-__global__ void __launch_bounds__(256)
-fusion_tail_kernel(const float* __restrict__ l0, const float* __restrict__ l1,
-                   const float* __restrict__ l2, const float* __restrict__ l3, int h0, int w0, int h1,
-                   int w1, int h2, int w2, int h3, int w3, const float* __restrict__ wf,
-                   const float* __restrict__ bf, float* __restrict__ out_nhwc,
-                   float* __restrict__ out_nchw, __nv_bfloat16* __restrict__ out_pad, int Cpad,
-                   int64_t total_px) {
-  // one warp per output pixel; lane = channel (C <= 32).  wT[k][co] keeps the 1x1 conv weights
-  // transposed so that lanes read consecutive banks.
-  constexpr int K = 4 * C;
-  __shared__ float wT[K][32];
-  __shared__ float cat[8][K];
-  for (int i = threadIdx.x; i < K * 32; i += 256) {
-    int k = i >> 5, co = i & 31;
-    wT[k][co] = co < C ? wf[co * K + k] : 0.f;
-  }
-  __syncthreads();
-  const int lane = threadIdx.x & 31, wid = threadIdx.x >> 5;
-  const float bias = lane < C ? bf[lane] : 0.f;
-  const int64_t hw = (int64_t)h0 * w0;
-  for (int64_t p = (int64_t)blockIdx.x * 8 + wid; p < total_px; p += (int64_t)gridDim.x * 8) {
-    const int ox = (int)(p % w0);
-    const int64_t t = p / w0;
-    const int oy = (int)(t % h0), b = (int)(t / h0);
-#pragma unroll
-    for (int lv = 0; lv < 4; ++lv) {
-      const float* src = lv == 0 ? l0 : lv == 1 ? l1 : lv == 2 ? l2 : l3;
-      const int hh = lv == 0 ? h0 : lv == 1 ? h1 : lv == 2 ? h2 : h3;
-      const int ww = lv == 0 ? w0 : lv == 1 ? w1 : lv == 2 ? w2 : w3;
-      float v = 0.f;
-      if (lane < C) {
-        int y0, y1, x0, x1;
-        float ly, lx;
-        bilinear_src(oy, (float)hh / h0, hh, y0, y1, ly);
-        bilinear_src(ox, (float)ww / w0, ww, x0, x1, lx);
-        const float* sb = src + (int64_t)b * hh * ww * C + lane;
-        v = (1.f - ly) * ((1.f - lx) * sb[((int64_t)y0 * ww + x0) * C] + lx * sb[((int64_t)y0 * ww + x1) * C]) +
-            ly * ((1.f - lx) * sb[((int64_t)y1 * ww + x0) * C] + lx * sb[((int64_t)y1 * ww + x1) * C]);
-        cat[wid][lv * C + lane] = v;
-      }
-    }
-    __syncwarp();
-    float acc = bias;
-#pragma unroll 8
-    for (int k = 0; k < K; ++k) acc = fmaf(wT[k][lane], cat[wid][k], acc);
-    __syncwarp();
-    if (lane < C) {
-      if (out_nhwc) out_nhwc[p * C + lane] = acc;
-      if (out_nchw) {
-        const int64_t bb = p / hw, r = p - bb * hw;
-        out_nchw[(bb * C + lane) * hw + r] = acc;
-      }
-    }
-    if (out_pad && lane < Cpad) out_pad[p * Cpad + lane] = __float2bfloat16_rn(lane < C ? acc : 0.f);
-  }
-}
-
-// Same head with the 1x1 fusion conv already applied per level (it commutes with the bilinear up-sample and
-// is folded into the head projections on the host): out[p] = bias + sum_lv bilinear_up(z_lv)[p].
+// ShapePropEncoder head with the 1x1 fusion conv already applied per level (it commutes with the bilinear up-sample
+// and is folded into the head projections on the host): out[p] = bias + sum_lv bilinear_up(z_lv)[p].
 // thread = (pixel, 4 channels); quads beyond C only zero-fill the padded bf16 copy.
 __global__ void __launch_bounds__(256)
 fusion_sum_kernel(const float* __restrict__ z0, const float* __restrict__ z1, const float* __restrict__ z2,
@@ -553,25 +493,6 @@ int dgtd_ln_rows_fwd(const float* y, const float* ln_w, const float* ln_b, void*
   int rc = ln_rows_any(y, ln_w, ln_b, out, out_dtype, rows, C, eps, (cudaStream_t)stream);
   if (rc) return rc;
   DGTD_LAUNCH_CHECK("ln_rows");
-  return 0;
-}
-
-int dgtd_fusion_head_fwd(const float* lv0, const float* lv1, const float* lv2, const float* lv3,
-                         const int* hw, const float* wf, const float* bf, float* out_nhwc,
-                         float* out_nchw, void* out_pad, int Cpad, int B, int C,
-                         dgtd_stream_t stream) {
-  DGTD_CHECK_ARG(lv0 && lv1 && lv2 && lv3 && hw && wf && bf, "fusion_head: null pointer");
-  DGTD_CHECK_ARG(C == 24, "fusion_head: latent dim %d not built (24 only, cod.py:1250)", C);
-  DGTD_CHECK_ARG(out_nhwc || out_nchw || out_pad, "fusion_head: no output requested");
-  DGTD_CHECK_ARG(!out_pad || Cpad >= C, "fusion_head: Cpad < C");
-  int64_t total = (int64_t)B * hw[0] * hw[1];
-  DGTD_CHECK_ARG(!out_pad || Cpad <= 32, "fusion_head: Cpad must be <= 32");
-  int blocks = cdiv(total, 8);
-  if (blocks > 148 * 16) blocks = 148 * 16;
-  fusion_tail_kernel<24><<<blocks, 256, 0, (cudaStream_t)stream>>>(
-      lv0, lv1, lv2, lv3, hw[0], hw[1], hw[2], hw[3], hw[4], hw[5], hw[6], hw[7], wf, bf, out_nhwc,
-      out_nchw, (__nv_bfloat16*)out_pad, Cpad, total);
-  DGTD_LAUNCH_CHECK("fusion_head");
   return 0;
 }
 

@@ -15,8 +15,8 @@
 //     operand.  One 4-D TMA box {64 ch, 24 px, 2 rows} per 64-channel block lands as 48 K rows x 128 B in the
 //     SWIZZLE_128B layout tcgen05.mma reads (zero fill outside the map == unfold's zero padding, cod.py:1204).
 //   * A is bf16 (kind::f16 wants both operands in ONE 16-bit format: an fp16 A against the bf16 X is an illegal
-//     instruction on sm_100a -- measured), K-major SWIZZLE_128B, RESIDENT in shared memory as seven 2-halo-row
-//     chunks (7 x 16 KB): the zero pattern of a row never changes, so per tile a builder thread (one per pixel)
+//     instruction on sm_100a -- measured), K-major SWIZZLE_32B, RESIDENT in shared memory as seven 2-halo-row
+//     chunks (7 x 12 KB): the zero pattern of a row never changes, so per tile a builder thread (one per pixel)
 //     only overwrites its 49 non-zeros.  Rounding the normalised weights to bf16 adds a zero-mean 2^-9 relative
 //     error per tap, i.e. ~2.5e-4 of max|y| after the 49-tap sum -- below the bf16 rounding of the stored result
 //     (2^-9 of the element) that bf16 storage implies anyway; stated tolerance 6e-3 of max|ref| per step.
@@ -42,20 +42,20 @@ constexpr int X_STAGE = (NB / 64) * XBLK;      // 24 KB
 constexpr int STG = 4 * 4096;                  // 4 epilogue warps x one staging tile (32 px x 128 B)
 constexpr int THREADS = 384;
 
-// Layout of the A (weights) operand in shared memory.  The kernel is bound by how many bytes of X it keeps in flight
-// (r2 profile: 72 KB per SM at ~2.8 us of loaded TMA latency = 3.8 TB/s of L2->SM traffic, tensor pipe 24 % busy),
-// so every KB not spent on A is a KB of X prefetch:
-//   SW128: rows of 128 B (96 used), SWIZZLE_128B K-major, 16 KB per chunk -> 4 X stages
-//   SW32 : one 4 KB block of 32-byte rows per K step, SWIZZLE_32B K-major, 12 KB per chunk -> 5 X stages
-//   RAWTMA: the 49 raw weights of the tile's pixels arrive as ONE TMA box {16 px, 8 rows, 49 taps} (25 KB, warp 3) instead
-//   of 49 global loads per builder thread.  fence.proxy.async compiles to MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC and the
-//   membar waits for every outstanding global load of the thread: with register prefetch the first publish of every
-//   tile stalled for a DRAM round trip (r2 profile: builder ~7900 cycles per tile against 2688 cycles of MMAs).
+// Shared-memory budget.  The kernel is bound by how many bytes of X it keeps in flight (r2 profile: 72 KB per SM at
+// ~2.8 us of loaded TMA latency = 3.8 TB/s of L2->SM traffic, tensor pipe 24 % busy), so every KB not spent elsewhere
+// is a KB of X prefetch.  The A (weights) operand is SWIZZLE_32B K-major: one 4 KB block of 128 rows x 32 B (16 K
+// columns) per K step, so a chunk takes 12 KB with no padding bytes, which leaves room for 5 X stages.
+// RAWTMA (taken when w % 4 == 0, see mp_tc_step_bf16): the 49 raw weights of the tile's pixels arrive as ONE TMA box
+// {16 px, 8 rows, 49 taps} (25 KB, warp 3) instead of 49 global loads per builder thread, and the slot costs one X
+// stage (4 stages).  fence.proxy.async compiles to MEMBAR.ALL.CTA + FENCE.VIEW.ASYNC and the membar waits for every
+// outstanding global load of the thread: with register prefetch the first publish of every tile stalled for a DRAM
+// round trip (r2 profile: builder ~7900 cycles per tile against 2688 cycles of MMAs).
 constexpr int W_BYTES = 49 * TH * TW * 4, W_SLOT = 25600;
-template <int SW, bool RAWTMA = false>
+template <bool RAWTMA>
 struct Cfg {
-  static constexpr int A_CHUNK = SW == 128 ? 128 * 128 : 3 * 128 * 32;
-  static constexpr int XSTAGES = (SW == 128 || RAWTMA) ? 4 : 5;
+  static constexpr int A_CHUNK = 3 * 128 * 32;
+  static constexpr int XSTAGES = RAWTMA ? 4 : 5;
   static constexpr int OFF_X = NCHUNK * A_CHUNK;
   static constexpr int OFF_STG = OFF_X + XSTAGES * X_STAGE;
   static constexpr int OFF_W = OFF_STG + STG;
@@ -64,12 +64,11 @@ struct Cfg {
   static constexpr int SMEM = OFF_BAR + NBARS * 8 + 16 + 1024;   // + alignment slack
   // byte offset of element (row m, chunk-local column kl) inside a chunk
   static __device__ __forceinline__ uint32_t a_off(uint32_t m, uint32_t kl) {
-    if (SW == 128) return m * 128 + ((((kl >> 3)) ^ (m & 7)) << 4) + ((kl & 7) << 1);
     return (kl >> 4) * 4096 + m * 32 + (((((kl >> 3) & 1)) ^ ((m >> 2) & 1)) << 4) + ((kl & 7) << 1);
   }
   // descriptor of K step k of chunk j, relative to the descriptor of the ring's first byte
   static __device__ __forceinline__ uint64_t a_desc_off(int j, int k) {
-    return (uint64_t)((j * A_CHUNK + (SW == 128 ? 32 * k : 4096 * k)) >> 4);
+    return (uint64_t)((j * A_CHUNK + 4096 * k) >> 4);
   }
 };
 
@@ -92,11 +91,11 @@ struct Params {
   float eps;
 };
 
-template <int SW, bool RAWTMA>
+template <bool RAWTMA>
 __global__ void __launch_bounds__(THREADS, 1)
 mp_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CUtensorMap tmOut,
              const __grid_constant__ CUtensorMap tmW, const Params p) {
-  using C = Cfg<SW, RAWTMA>;
+  using C = Cfg<RAWTMA>;
   constexpr int A_CHUNK = C::A_CHUNK, XSTAGES = C::XSTAGES, OFF_X = C::OFF_X, OFF_STG = C::OFF_STG, OFF_BAR = C::OFF_BAR;
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~(uintptr_t)1023);
@@ -202,7 +201,7 @@ mp_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CU
     // descriptors are precomputed and the chunk loop is unrolled (r2 profile: the first version spent 2/3 of the
     // issuing warp's time on loop overhead and ran the tensor pipe at 24 %).
     constexpr uint32_t IDESC = idesc();
-    const uint64_t da0 = bw::umma_smem_desc_kmajor(bw::smem_u32(sA), SW);
+    const uint64_t da0 = bw::umma_smem_desc_kmajor(bw::smem_u32(sA), 32);
     const uint64_t db0 = bw::umma_smem_desc_mnmajor_sw128(bw::smem_u32(sX), XBLK, 1024);
     int stage = 0, iter = 0;
     uint32_t phase = 0, tphase = 0;
@@ -392,26 +391,25 @@ mp_tc_kernel(const __grid_constant__ CUtensorMap tmX, const __grid_constant__ CU
 }  // namespace mptc
 
 // One diffusion step on the tensor pipe; 0 on success, 1 when the shape is not handled here.
-template <int SW, bool RAWTMA>
+template <bool RAWTMA>
 static int mp_tc_launch(const CUtensorMap& tmX, const CUtensorMap& tmOut, const CUtensorMap& tmW, const mptc::Params& p,
                         int grid, cudaStream_t s) {
   using namespace mptc;
-  using Cf = Cfg<SW, RAWTMA>;
+  using Cf = Cfg<RAWTMA>;
   static bool configured = false;
   if (!configured) {
-    cudaError_t e1 = cudaFuncSetAttribute(mp_tc_kernel<SW, RAWTMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cf::SMEM);
+    cudaError_t e1 = cudaFuncSetAttribute(mp_tc_kernel<RAWTMA>, cudaFuncAttributeMaxDynamicSharedMemorySize, Cf::SMEM);
     if (e1 != cudaSuccess) {
       set_error("message_passing_tc: cannot opt in to %d B smem: %s", Cf::SMEM, cudaGetErrorString(e1));
       return -2;
     }
     configured = true;
   }
-  mp_tc_kernel<SW, RAWTMA><<<grid, THREADS, Cf::SMEM, s>>>(tmX, tmOut, tmW, p);
+  mp_tc_kernel<RAWTMA><<<grid, THREADS, Cf::SMEM, s>>>(tmX, tmOut, tmW, p);
   return 0;
 }
 
-int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h, int w, int c, float eps, int variant,
-                    cudaStream_t s) {
+int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h, int w, int c, float eps, cudaStream_t s) {
   using namespace mptc;
   if (c % NB != 0 || (int64_t)h * w * 49 >= (int64_t)1 << 31) return 1;
   CUtensorMap tmX, tmOut;
@@ -431,7 +429,7 @@ int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h,
   p.eps = eps;
   const int grid = p.num_tiles < sm_count() ? p.num_tiles : sm_count();
   CUtensorMap tmW = tmX;   // placeholder when the raw weights are read with plain loads
-  const bool rawtma = variant == 0 && w % 4 == 0;   // TMA needs 16-byte multiples for the weight planes' row pitch
+  const bool rawtma = w % 4 == 0;   // TMA needs 16-byte multiples for the weight planes' row pitch
   if (rawtma) {
     const uint64_t wdims[4] = {(uint64_t)w, (uint64_t)h, 49, (uint64_t)n};
     const uint64_t wstr[3] = {(uint64_t)w * 4, (uint64_t)h * w * 4, (uint64_t)49 * h * w * 4};
@@ -439,8 +437,7 @@ int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h,
     rc = make_tmap(&tmW, weight, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, wdims, wstr, wbox, CU_TENSOR_MAP_SWIZZLE_NONE);
     if (rc) return rc;
   }
-  if (variant == 1) return mp_tc_launch<128, false>(tmX, tmOut, tmW, p, grid, s);
-  return rawtma ? mp_tc_launch<32, true>(tmX, tmOut, tmW, p, grid, s) : mp_tc_launch<32, false>(tmX, tmOut, tmW, p, grid, s);
+  return rawtma ? mp_tc_launch<true>(tmX, tmOut, tmW, p, grid, s) : mp_tc_launch<false>(tmX, tmOut, tmW, p, grid, s);
 }
 
 }  // namespace dgtd

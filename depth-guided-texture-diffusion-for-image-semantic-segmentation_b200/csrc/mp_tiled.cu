@@ -192,8 +192,7 @@ static int mp_step(const void* x, const float* weight, void* out, int n, int h, 
 }
 
 // mp_tc.cu: one step on the tensor pipe (banded GEMM); returns 1 when the shape is not handled there
-int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h, int w, int c, float eps, int variant,
-                    cudaStream_t s);
+int mp_tc_step_bf16(const void* x, const float* weight, void* out, int n, int h, int w, int c, float eps, cudaStream_t s);
 // mp_tc_f32.cu: the same step for fp32 storage (three bf16 products, fp32-level accuracy)
 int mp_tc_step_f32(const void* x, const float* weight, void* out, int n, int h, int w, int c, float eps, cudaStream_t s);
 
@@ -202,10 +201,9 @@ int mp_tc_step_f32(const void* x, const float* weight, void* out, int n, int h, 
 using namespace dgtd;
 
 extern "C" int dgtd_message_passing_tc_fwd(const void* x, const float* weight, void* out, void* tmp, int n, int h, int w,
-                                           int c, int T, float eps, int dtype, int flags, dgtd_stream_t stream) {
+                                           int c, int T, float eps, int dtype, dgtd_stream_t stream) {
   DGTD_CHECK_ARG(x && weight && out, "message_passing_tc: null pointer");
   DGTD_CHECK_ARG(dtype == DGTD_BF16 || dtype == DGTD_F32, "message_passing_tc: bad dtype %d", dtype);
-  DGTD_CHECK_ARG(flags == 0 || flags == 1, "message_passing_tc: unknown flags %d", flags);
   DGTD_CHECK_ARG(n > 0 && h > 0 && w > 0 && c >= 256 && c % 256 == 0 && T >= 1,
                  "message_passing_tc: bad shape n=%d h=%d w=%d c=%d T=%d (c must be a multiple of 256)", n, h, w, c, T);
   DGTD_CHECK_ARG(T == 1 || tmp, "message_passing_tc: tmp buffer required for T > 1");
@@ -216,7 +214,7 @@ extern "C" int dgtd_message_passing_tc_fwd(const void* x, const float* weight, v
   const void* src = x;   // ping-pong so that the last step lands in `out`
   for (int t = 0; t < T; ++t) {
     void* dst = ((T - 1 - t) % 2 == 0) ? out : tmp;
-    int rc = dtype == DGTD_BF16 ? mp_tc_step_bf16(src, weight, dst, n, h, w, c, eps, flags & 1, s)
+    int rc = dtype == DGTD_BF16 ? mp_tc_step_bf16(src, weight, dst, n, h, w, c, eps, s)
                                 : mp_tc_step_f32(src, weight, dst, n, h, w, c, eps, s);
     if (rc > 0) {
       set_error("message_passing_tc: shape not supported");
@@ -256,7 +254,7 @@ static int mp_tiled_simt(const void* x, const float* weight, void* out, void* tm
                  "message_passing_tiled: buffers must be 16-byte aligned");
   // bf16 storage with C % 256 == 0 runs on the tensor pipe (mp_tc.cu); everything else on the SIMT kernel below
   if (allow_tc && c % 256 == 0 && (int64_t)h * w * 49 < ((int64_t)1 << 31) && (dtype == DGTD_BF16 || w % 4 == 0))
-    return dgtd_message_passing_tc_fwd(x, weight, out, tmp, n, h, w, c, T, eps, dtype, 0, stream);
+    return dgtd_message_passing_tc_fwd(x, weight, out, tmp, n, h, w, c, T, eps, dtype, stream);
   cudaStream_t s = (cudaStream_t)stream;
   const void* src = x;   // ping-pong so that the last step lands in `out`
   for (int t = 0; t < T; ++t) {

@@ -335,14 +335,14 @@ int tc_gemm2_ln_launch(const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16*
 }
 
 // Split-K partial products for weight gradients: partial[z] (M x N fp32) = A[:, Kz] . B[:, Kz]^T
-// partial: splits x roundup(M, 256) x N floats.  mn_major: A is (K x M), B is (K x N) row-major.
+// partial: splits x roundup(M, 256) x N floats.  A is (K x M), B is (K x N) row-major, read as MN-major operands.
 int tc_gemm2_splitk(const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16* B, int64_t ldb, float* partial, int M,
-                    int N, int K, int splits, int mn_major, cudaStream_t s) {
+                    int N, int K, int splits, cudaStream_t s) {
   TcParams p{};
   p.M = M; p.N = N; p.K = K; p.out = partial; p.ldo = N; p.rows_per_sample = 1;
   p.splits = splits;
   p.split_rows = cdiv(M, 256) * 256;
-  p.mn_major = mn_major;
+  p.mn_major = 1;
   const int num_kb = cdiv(K, 64);
   p.kb_per_split = cdiv(num_kb, splits);
   if ((int64_t)(splits - 1) * p.kb_per_split >= num_kb) {   // every split must own at least one k-block

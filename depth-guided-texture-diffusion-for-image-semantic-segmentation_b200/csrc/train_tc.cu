@@ -241,7 +241,7 @@ __global__ void sum_parts_kernel(const float* __restrict__ part, float* __restri
 }
 
 int tc_gemm2_splitk(const __nv_bfloat16* A, int64_t lda, const __nv_bfloat16* B, int64_t ldb, float* partial, int M,
-                    int N, int K, int splits, int mn_major, cudaStream_t s);
+                    int N, int K, int splits, cudaStream_t s);
 
 }  // namespace dgtd
 
@@ -354,8 +354,8 @@ int dgtd_colsum_bf16(const void* x, float* ws, float* out, int M, int N, dgtd_st
   return 0;
 }
 
-// out = aT[Mo, Kr] . bT[No, Kr]^T  (fp32), reduction over the long Kr axis split across CTA pairs.
-// transpose_out != 0 writes out as (No x Mo).  ws: dgtd_wgrad_tc_ws_floats floats.
+// Weight gradients (Mo x No fp32) reduce over the long Kr axis: it is split across CTA pairs and the partial products
+// are summed in a fixed order.  ws: dgtd_wgrad_tc_ws_floats floats.
 static int wgrad_splits(int Mo, int No, int Kr) {
   const int tiles = cdiv(Mo, 256) * cdiv(No, No % 256 == 0 ? 256 : 128);
   int s = cdiv(148, tiles);
@@ -368,29 +368,9 @@ static int wgrad_splits(int Mo, int No, int Kr) {
 }
 int dgtd_wgrad_tc_ws_floats(int Mo, int No, int Kr) { return wgrad_splits(Mo, No, Kr) * cdiv(Mo, 256) * 256 * No; }
 
-static int wgrad_tc_run(const void* a, int64_t lda, const void* b, int64_t ldb, float* out, float* ws, int Mo, int No,
-                        int Kr, int transpose_out, int mn_major, cudaStream_t s) {
-  const int S = wgrad_splits(Mo, No, Kr);
-  int rc = tc_gemm2_splitk((const __nv_bfloat16*)a, lda, (const __nv_bfloat16*)b, ldb, ws, Mo, No, Kr, S, mn_major, s);
-  if (rc) return rc;
-  DGTD_LAUNCH_CHECK("wgrad_tc");
-  const int64_t n = (int64_t)Mo * No;
-  sum_parts_kernel<<<cdiv(n, 256), 256, 0, s>>>(ws, out, n, S, (int64_t)cdiv(Mo, 256) * 256 * No,
-                                                transpose_out ? Mo : 0, No);
-  DGTD_LAUNCH_CHECK("wgrad_tc.reduce");
-  return 0;
-}
-
-int dgtd_wgrad_tc(const void* aT, const void* bT, float* out, float* ws, int Mo, int No, int Kr, int transpose_out,
-                  dgtd_stream_t stream) {
-  DGTD_CHECK_ARG(aT && bT && out && ws, "wgrad_tc: null pointer");
-  DGTD_CHECK_ARG(Mo >= 8 && No >= 8 && No % 8 == 0 && Kr >= 64 && Kr % 8 == 0,
-                 "wgrad_tc: need No %% 8 == 0, Kr %% 8 == 0, Kr >= 64 (got %d, %d, %d)", Mo, No, Kr);
-  return wgrad_tc_run(aT, Kr, bT, Kr, out, ws, Mo, No, Kr, transpose_out, 0, (cudaStream_t)stream);
-}
-
-// Same product from UN-transposed operands: out (Mo x No) = a[Kr, Mo]^T . b[Kr, No], a and b row-major
+// Weight gradient from UN-transposed operands: out (Mo x No) = a[Kr, Mo]^T . b[Kr, No], a and b row-major
 // activation matrices (pitches lda / ldb elements, column slices allowed), read as MN-major UMMA operands.
+// transpose_out != 0 writes out as (No x Mo).
 int dgtd_wgrad_tc_mn(const void* a, int lda, const void* b, int ldb, float* out, float* ws, int Mo, int No, int Kr,
                      int transpose_out, dgtd_stream_t stream) {
   DGTD_CHECK_ARG(a && b && out && ws, "wgrad_tc_mn: null pointer");
@@ -400,7 +380,16 @@ int dgtd_wgrad_tc_mn(const void* a, int lda, const void* b, int ldb, float* out,
                  lda, ldb);
   DGTD_CHECK_ARG(((reinterpret_cast<uintptr_t>(a) | reinterpret_cast<uintptr_t>(b)) & 15) == 0,
                  "wgrad_tc_mn: operands must be 16-byte aligned");
-  return wgrad_tc_run(a, lda, b, ldb, out, ws, Mo, No, Kr, transpose_out, 1, (cudaStream_t)stream);
+  cudaStream_t s = (cudaStream_t)stream;
+  const int S = wgrad_splits(Mo, No, Kr);
+  int rc = tc_gemm2_splitk((const __nv_bfloat16*)a, lda, (const __nv_bfloat16*)b, ldb, ws, Mo, No, Kr, S, s);
+  if (rc) return rc;
+  DGTD_LAUNCH_CHECK("wgrad_tc");
+  const int64_t n = (int64_t)Mo * No;
+  sum_parts_kernel<<<cdiv(n, 256), 256, 0, s>>>(ws, out, n, S, (int64_t)cdiv(Mo, 256) * 256 * No,
+                                                transpose_out ? Mo : 0, No);
+  DGTD_LAUNCH_CHECK("wgrad_tc.reduce");
+  return 0;
 }
 
 }  // extern "C"

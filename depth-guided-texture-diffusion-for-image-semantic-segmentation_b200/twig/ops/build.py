@@ -27,7 +27,7 @@ LIB = os.path.join(HERE, "libdgtd_ops.so")
 
 NVCC_FLAGS = [
     "-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
-    "--use_fast_math" if False else "-Xptxas=-v",
+    "-Xptxas=-v",
     "-Xcompiler", "-fPIC", "-Xcompiler", "-O3",
 ]
 

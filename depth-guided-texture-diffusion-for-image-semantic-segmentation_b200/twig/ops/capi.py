@@ -34,7 +34,7 @@ SIGNATURES = {
     "dgtd_message_passing_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],
     "dgtd_message_passing_tiled_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _I, _P],
     "dgtd_message_passing_tiled_simt_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _I, _P],
-    "dgtd_message_passing_tc_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _I, _I, _P],
+    "dgtd_message_passing_tc_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _I, _P],
     "dgtd_pack_regressor": [_P, _P, _P, _I, _P],
     "dgtd_message_passing_regress_fwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _I, _I, _P],
     "dgtd_message_passing_bwd": [_P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _F, _P],
@@ -54,7 +54,6 @@ SIGNATURES = {
     "dgtd_linear_lnfold_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _I, _I, _P],
     "dgtd_linear_residual_fwd": [_P, _P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _I, _P],
     "dgtd_convnext_mlp_fused_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _L, _I, _P],
-    "dgtd_fusion_head_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
     "dgtd_fusion_sum_fwd": [_P, _P, _P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
     "dgtd_conv_nhwc_fwd": [_P, _P, _P, _P] + [_I] * 15 + [_P],
     "dgtd_conv_nhwc_grouped_fwd": [_P, _P, _P, _P] + [_I] * 16 + [_L, _I, _L, _P],
@@ -79,7 +78,6 @@ SIGNATURES = {
     "dgtd_colsum_bf16": [_P, _P, _P, _I, _I, _P],
     "dgtd_eltwise_colsum_ws_floats": [_I, _I],
     "dgtd_eltwise_colsum": [_P, _P, _P, _P, _I, _P, _P, _I, _I, _I, _P],
-    "dgtd_wgrad_tc": [_P, _P, _P, _P, _I, _I, _I, _I, _P],
     "dgtd_wgrad_tc_ws_floats": [_I, _I, _I],
     "dgtd_wgrad_tc_mn": [_P, _I, _P, _I, _P, _P, _I, _I, _I, _I, _P],
     "dgtd_ln_rows_fwd": [_P, _P, _P, _P, _I, _L, _I, _F, _P],

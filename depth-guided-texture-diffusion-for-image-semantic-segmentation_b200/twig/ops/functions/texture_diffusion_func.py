@@ -20,7 +20,7 @@ from ..capi import ACT_GELU, ACT_NONE, ACT_RELU, BF16, F32, call, check_cuda, pt
 __all__ = [
     "surface_normals", "HighpassPlan", "fft_highpass", "diffusion_front", "MessagePassingFunction",
     "message_passing_core", "message_passing_tiled", "conv1x1_nchw_autograd", "resize_bilinear_nchw_autograd", "conv1x1_nchw", "resize_nchw", "layer_norm",
-    "stem", "stem_patches", "ln_rows_", "fusion_sum", "ln_patchify", "dwconv7_ln", "dwconv7_ln_tma", "linear", "linear_ln", "linear_tf32", "linear_residual_", "fusion_head", "conv_nhwc", "conv_nhwc_grouped",
+    "stem", "stem_patches", "ln_rows_", "fusion_sum", "ln_patchify", "dwconv7_ln", "dwconv7_ln_tma", "linear", "linear_ln", "linear_tf32", "linear_residual_", "conv_nhwc", "conv_nhwc_grouped",
     "resize_nhwc", "cast", "nhwc_to_nchw", "nchw_to_nhwc", "enable_gemm_profile", "collect_gemm_profile",
 ]
 
@@ -256,15 +256,14 @@ def resize_bilinear_nchw_autograd(x, size):
 
 def message_passing_tiled(x: torch.Tensor, weight: torch.Tensor, steps: int, eps: float = 1e-5, impl: str = "auto"):
     """Large-map variant: x (n,h,w,c) channels-last storage (fp32|bf16), weight (n,49,h,w) fp32.
-    impl: "auto" (tensor-pipe banded GEMM when the shape qualifies, else the SIMT kernel), "simt", "tc",
-    "tc_sw128" (weights operand in SWIZZLE_128B rows instead of the compact SWIZZLE_32B blocks)."""
+    impl: "auto" (tensor-pipe banded GEMM when the shape qualifies, else the SIMT kernel), "simt", "tc"."""
     check_cuda(x, weight)
     n, h, w, c = x.shape
     out = torch.empty_like(x)
     tmp = torch.empty_like(x) if steps > 1 else None
-    if impl in ("tc", "tc_sw128"):
+    if impl == "tc":
         call("dgtd_message_passing_tc_fwd", ptr(x), ptr(weight), ptr(out), ptr(tmp), n, h, w, c, steps,
-             float(eps), capi.dtype_code(x.dtype), 1 if impl == "tc_sw128" else 0, stream())
+             float(eps), capi.dtype_code(x.dtype), stream())
         return out
     assert impl in ("auto", "simt")
     call("dgtd_message_passing_tiled_fwd" if impl == "auto" else "dgtd_message_passing_tiled_simt_fwd", ptr(x),
@@ -476,22 +475,6 @@ def convnext_mlp_fused_(y: torch.Tensor, row_stats: torch.Tensor, w1: torch.Tens
 
 
 # ------------------------------------------------------------------------------------------ a9
-def fusion_head(levels: List[torch.Tensor], hw: List[Tuple[int, int]], wf, bf, B: int, want_nhwc=True,
-                want_nchw=False, pad_to: int = 0):
-    """levels[i]: (B*h_i*w_i, C) fp32 projections.  Returns (nhwc, nchw, padded-bf16) tensors."""
-    check_cuda(*levels, wf, bf)
-    C = wf.shape[0]
-    dev = levels[0].device
-    h0, w0 = hw[0]
-    nhwc = torch.empty(B, h0, w0, C, device=dev, dtype=torch.float32) if want_nhwc else None
-    nchw = torch.empty(B, C, h0, w0, device=dev, dtype=torch.float32) if want_nchw else None
-    pad = torch.empty(B, h0, w0, pad_to, device=dev, dtype=torch.bfloat16) if pad_to else None
-    hw_arr = (capi.c_int * 8)(*[v for pair in hw for v in pair])
-    call("dgtd_fusion_head_fwd", ptr(levels[0]), ptr(levels[1]), ptr(levels[2]), ptr(levels[3]), hw_arr,
-         ptr(wf), ptr(bf), ptr(nhwc), ptr(nchw), ptr(pad), pad_to, B, C, stream())
-    return nhwc, nchw, pad
-
-
 def fusion_sum(levels: List[torch.Tensor], hw: List[Tuple[int, int]], bias, B: int, want_nhwc=True,
                want_nchw=False, pad_to: int = 0):
     """levels[i]: (B*h_i*w_i, C) fp32 with the fusion conv already folded in; out = bias + sum_i up(levels[i]).

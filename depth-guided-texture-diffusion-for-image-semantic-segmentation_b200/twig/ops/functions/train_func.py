@@ -116,19 +116,9 @@ def eltwise_colsum(src, mode, aux=None, keep=None, rows_per_sample=1):
     return dst, out
 
 
-def wgrad_tc(aT, bT, transpose_out=False):
-    """(Mo x No) = aT[Mo,Kr] @ bT[No,Kr]^T on tcgen05 (split-K over Kr); fp32 result (optionally transposed)."""
-    Mo, Kr = aT.shape
-    No = bT.shape[0]
-    out = _empty((No, Mo) if transpose_out else (Mo, No), aT)
-    ws = _empty((capi.load().dgtd_wgrad_tc_ws_floats(Mo, No, Kr),), aT)
-    call("dgtd_wgrad_tc", ptr(aT), ptr(bT), ptr(out), ptr(ws), Mo, No, Kr, int(transpose_out), stream())
-    return out
-
-
 def wgrad_tc_mn(a, b, transpose_out=False):
-    """(Mo x No) = a[Kr,Mo]^T @ b[Kr,No] on tcgen05 straight from row-major bf16 activations (column
-    slices allowed: stride(0) = pitch, stride(1) = 1); fp32 result (optionally transposed)."""
+    """(Mo x No) = a[Kr,Mo]^T @ b[Kr,No] on tcgen05 (split-K over Kr) straight from row-major bf16 activations
+    (column slices allowed: stride(0) = pitch, stride(1) = 1); fp32 result (optionally transposed)."""
     Kr, Mo = a.shape
     No = b.shape[1]
     assert b.shape[0] == Kr and a.stride(1) == 1 and b.stride(1) == 1

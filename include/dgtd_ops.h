@@ -100,10 +100,9 @@ int dgtd_message_passing_tiled_simt_fwd(const void* x, const float* weight, void
 /* The same operator (cod.py:1201-1205, shared weights) on the TENSOR pipe: per 8x16-pixel tile the step is the
  * banded GEMM Y[128 px, c] = A[128, 336 halo px] . X[336, c] on tcgen05.mma; A holds the 49 normalised weights of
  * each pixel in bf16, X is the NHWC map read through TMA as an MN-major operand.  bf16 storage, c a multiple
- * of 256.  flags: 0 = weights operand in the compact SWIZZLE_32B layout (5 X stages in flight), 1 = SWIZZLE_128B rows
- * (4 stages; A/B variant of the same kernel).  dgtd_message_passing_tiled_fwd dispatches here when the shape qualifies. */
+ * of 256.  dgtd_message_passing_tiled_fwd dispatches here when the shape qualifies. */
 int dgtd_message_passing_tc_fwd(const void* x, const float* weight, void* out, void* tmp,
-                                int n, int h, int w, int c, int T, float eps, int dtype, int flags,
+                                int n, int h, int w, int c, int T, float eps, int dtype,
                                 dgtd_stream_t stream);
 /* Same operator with the MODEL's per-channel weights generated on chip (SURVEY.md 8d config 4, mode W2):
  * W[c,k,p] = sigmoid(Wr[c*49+k,:] . guide[:,p] + br[c*49+k]) (ShapePropWeightRegressor, cod.py:1051-1060,
@@ -206,16 +205,11 @@ int dgtd_linear_residual_fwd(const void* a, const void* w, const float* bias, co
                              float* out, int M, int N, int K, int dtype_in, dgtd_stream_t stream);
 
 /* ---- a9: ShapePropEncoder head, cod.py:1171-1176 ------------------------------------------ */
-/* lv[i]: level-i projection (B*h_i*w_i, C) fp32 (output of the per-level 1x1 conv);
- * bilinear up to (h_0,w_0), concat, 1x1 conv (wf: C x 4C, bf: C).  Writes any of:
- * out_nhwc (B,h0,w0,C) fp32, out_nchw (B,C,h0,w0) fp32, out_pad (B,h0,w0,Cpad) bf16 zero
- * padded to Cpad channels (operand of the tensor-core decoders).  hw = {h0,w0,...,h3,w3}. */
-int dgtd_fusion_head_fwd(const float* lv0, const float* lv1, const float* lv2, const float* lv3,
-                         const int* hw, const float* wf, const float* bf, float* out_nhwc,
-                         float* out_nchw, void* out_pad, int Cpad, int B, int C,
-                         dgtd_stream_t stream);
-/* Same head after folding the fusion conv into the four head projections (a 1x1 conv commutes with the
- * bilinear up-sample): z_i (B*h_i*w_i, C) fp32 = x_i (Wf_i Wh_i)^T + Wf_i bh_i;  out = bias + sum_i up(z_i). */
+/* Per-level 1x1 projections, bilinear up to (h0,w0), concat and 1x1 fusion conv, with the fusion conv folded into
+ * the four head projections (a 1x1 conv commutes with the bilinear up-sample):
+ * z_i (B*h_i*w_i, C) fp32 = x_i (Wf_i Wh_i)^T + Wf_i bh_i;  out = bias + sum_i up(z_i).  hw = {h0,w0,...,h3,w3}.
+ * Writes any of: out_nhwc (B,h0,w0,C) fp32, out_nchw (B,C,h0,w0) fp32, out_pad (B,h0,w0,Cpad) bf16 zero padded
+ * to Cpad channels (operand of the tensor-core decoders).  C and Cpad multiples of 4. */
 int dgtd_fusion_sum_fwd(const float* z0, const float* z1, const float* z2, const float* z3, const int* hw,
                         const float* bias, float* out_nhwc, float* out_nchw, void* out_pad, int Cpad, int B, int C,
                         dgtd_stream_t stream);
@@ -305,14 +299,11 @@ int dgtd_colsum_bf16(const void* x, float* ws, float* out, int M, int N, dgtd_st
 int dgtd_eltwise_colsum_ws_floats(int M, int N);
 int dgtd_eltwise_colsum(const void* src, const void* aux, void* dst, const float* keep, int rows_per_sample, float* ws,
                         float* colsum, int M, int N, int mode, dgtd_stream_t stream);
-/* out (Mo x No fp32, or its transpose) = aT[Mo,Kr] . bT[No,Kr]^T: weight gradient on tcgen05 with
- * split-K over the long row axis Kr + fixed-order reduction.  ws: dgtd_wgrad_tc_ws_floats floats. */
-int dgtd_wgrad_tc(const void* aT, const void* bT, float* out, float* ws, int Mo, int No, int Kr, int transpose_out,
-                  dgtd_stream_t stream);
-int dgtd_wgrad_tc_ws_floats(int Mo, int No, int Kr);
-/* Same product from UN-transposed operands: out (Mo x No) = a[Kr,Mo]^T . b[Kr,No], a / b row-major bf16
+/* Weight gradient on tcgen05: out (Mo x No fp32, or its transpose) = a[Kr,Mo]^T . b[Kr,No], a / b row-major bf16
  * activation matrices (pitches lda / ldb in elements; column slices allowed), consumed as MN-major tcgen05
- * operands -- the weight gradient dW = dY^T X straight from dY and X.  ws as for dgtd_wgrad_tc. */
+ * operands -- dW = dY^T X straight from dY and X.  Split-K over the long row axis Kr + fixed-order reduction.
+ * ws: dgtd_wgrad_tc_ws_floats(Mo, No, Kr) floats. */
+int dgtd_wgrad_tc_ws_floats(int Mo, int No, int Kr);
 int dgtd_wgrad_tc_mn(const void* a, int lda, const void* b, int ldb, float* out, float* ws, int Mo, int No, int Kr,
                      int transpose_out, dgtd_stream_t stream);
 /* Decoder-bank backward, data-movement halves (ShapePropDecoder cod.py:1210-1226 + folded injection :1471).

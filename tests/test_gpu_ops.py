@@ -197,26 +197,24 @@ def test_message_passing_regress_at_microbench_size(OP, storage, T):
 
 @pytest.mark.parametrize("n,h,w,c,T", [(1, 40, 70, 256, 1), (2, 17, 33, 256, 3), (1, 64, 64, 512, 2), (1, 8, 16, 256, 1),
                                        (1, 5, 3, 256, 2), (3, 23, 16, 256, 1), (2, 200, 264, 256, 2)])
-@pytest.mark.parametrize("impl", ["tc", "tc_sw128"])
-def test_message_passing_tensor_core_banded_gemm(OP, n, h, w, c, T, impl):
+def test_message_passing_tensor_core_banded_gemm(OP, n, h, w, c, T):
     """mp_tc.cu: the step as Y[128 px, C] = A[128, 336] . X[336, C] on tcgen05 (bf16 storage).  Ragged maps (tiles
     clipped by TMA on both axes), maps smaller than one tile, two channel passes (C = 512), several images, T > 1.
     The last case has 850 tiles (> 148 CTAs: every CTA walks several tiles, the A ring is rewritten in flight).
     Stated tolerance 6e-3 * T of max|ref|: one bf16 rounding of the stored result per step (2^-9 of the element)
-    plus the bf16 rounding of the normalised weights in the A operand (zero-mean, ~1e-3 of max|ref| at 4.5 sigma).
-    impl "tc" = compact SWIZZLE_32B weights operand (shipped), "tc_sw128" = SWIZZLE_128B rows (A/B variant)."""
+    plus the bf16 rounding of the normalised weights in the A operand (zero-mean, ~1e-3 of max|ref| at 4.5 sigma)."""
     g = torch.Generator().manual_seed(23)
     x = torch.randn(n, c, h, w, generator=g).to(torch.bfloat16)
     wgt = torch.rand(n, 49, h, w, generator=g)
     ref = O.message_passing_core(x.double(), wgt.double(), 7, T)
     xc = x.permute(0, 2, 3, 1).contiguous().cuda()
-    got = OP.message_passing_tiled(xc, wgt.cuda(), T, impl=impl)
+    got = OP.message_passing_tiled(xc, wgt.cuda(), T, impl="tc")
     assert got.dtype == torch.bfloat16
     err = check(got.float().permute(0, 3, 1, 2), ref, 6e-3 * T)
     simt = OP.message_passing_tiled(xc, wgt.cuda(), T, impl="simt") if c % 128 == 0 else None
     if simt is not None:      # the CUDA-core kernel of the same operator (fp32 weights): two independently bf16-rounded results
         d = float((got.float() - simt.float()).abs().max() / ref.abs().max())
-        print(f"tc[{impl}] vs oracle {err:.2e}; vs SIMT kernel {d:.2e}")
+        print(f"tc vs oracle {err:.2e}; vs SIMT kernel {d:.2e}")
         assert d <= 1e-2 * T
 
 
@@ -409,7 +407,10 @@ def test_convnext_block_fp32_vs_reference_golden(golden_ops):
     check(y, t64(golden_ops["blk_out"]), 2e-5)
 
 
-def test_fusion_head(OP):
+def test_fusion_sum(OP):
+    """ShapePropEncoder head (cod.py:1171-1176) with the 1x1 fusion conv folded into the level projections, as
+    `_head` calls it: z_i = lv_i Wf_i^T per level, then bias + sum_i bilinear_up(z_i) against the un-folded
+    conv2d(cat(bilinear_up(lv_i)), Wf, bf)."""
     g = torch.Generator().manual_seed(11)
     B, C = 2, 24
     hw = [(24, 20), (12, 10), (6, 5), (3, 3)]
@@ -417,9 +418,10 @@ def test_fusion_head(OP):
     wf, bf = torch.randn(C, 4 * C, 1, 1, generator=g) * 0.2, torch.randn(C, generator=g)
     cat = torch.cat([O.bilinear_resize(v.double(), hw[0]) for v in lv], 1)
     ref = F.conv2d(cat, wf.double(), bf.double())
-    lv_rows = [v.permute(0, 2, 3, 1).reshape(-1, C).contiguous().cuda() for v in lv]
-    nhwc, nchw, pad = OP.fusion_head(lv_rows, hw, wf.reshape(C, 4 * C).cuda().contiguous(), bf.cuda(), B,
-                                     want_nhwc=True, want_nchw=True, pad_to=32)
+    wf2 = wf.reshape(C, 4 * C).double()
+    z = [(v.double().permute(0, 2, 3, 1).reshape(-1, C) @ wf2[:, i * C:(i + 1) * C].T).float().contiguous().cuda()
+         for i, v in enumerate(lv)]
+    nhwc, nchw, pad = OP.fusion_sum(z, hw, bf.cuda(), B, want_nhwc=True, want_nchw=True, pad_to=32)
     check(nchw, ref, 1e-5)
     check(nhwc.permute(0, 3, 1, 2), ref, 1e-5)
     check(pad[..., :C].float().permute(0, 3, 1, 2), ref, 1e-2)   # bf16 storage

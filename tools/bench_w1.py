@@ -17,7 +17,7 @@ def t(fn, n=5):
     for _ in range(n): fn()
     b.record(); torch.cuda.synchronize()
     return a.elapsed_time(b) / n
-for impl in sys.argv[1:] or ["tc", "tc_sw128", "simt"]:
+for impl in sys.argv[1:] or ["tc", "simt"]:
     for T in (1, 4):
         ms = t(lambda: OP.message_passing_tiled(xb, wgt, T, impl=impl))
         nbytes = (2 * C * 2 + 49 * 4) * S * S
