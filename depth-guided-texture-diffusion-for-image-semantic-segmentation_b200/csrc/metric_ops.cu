@@ -6,7 +6,8 @@
 // count / foreground index sums per image; pass 2 accumulates, per centroid quadrant, the integer moments
 // S(d), S(g), S(d^2), S(d g), S(d^2 g) of d = pred_u8 - min; a one-thread-per-image tail evaluates both metrics in
 // float64 from the exact integers (variances as N*S2 - S1^2: no cancellation).  No atomics, no floating-point
-// reduction: results are bit-stable and independent of the launch geometry.
+// reduction: results are bit-stable and independent of the launch geometry.  The weighted F-measure (below
+// metric_curves_kernel) reuses the quantise and info passes and adds an exact Euclidean distance transform.
 #include "common.cuh"
 
 namespace dgtd {
@@ -314,6 +315,214 @@ __global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchu
   }
 }
 
+// ---- weighted F-measure (pysodmetrics `WeightedFmeasure.cal_wfm`, beta = 1) -----------------------------------------
+// After the quantise and info passes above: (1) a table pass evaluates E = |p(u) - g| for both labels; (2) a column
+// pass finds, per pixel, the nearest foreground row in its column (the lower row on a tie); (3) a row pass takes the
+// lower envelope of the parabolas (x - j)^2 + dy_j^2 (Meijster et al. 2000, exact integer separators; the lower
+// column on a tie), writes the u8 prediction of the nearest foreground pixel (Et, transposed) and sums the
+// distance-weighted background errors of the row; (4) a tile pass applies the 7x7 Gaussian to Et at the foreground
+// pixels and sums min(E, EA) per tile; (5) a per-image tail.  The two-pass tie rules make the nearest pixel the one
+// with the least (squared distance, column, row): SciPy's `distance_transform_edt(return_indices=True)`.
+// Row / column indices are int32 and squared distances int64 (H * W < 2^28).  No floating-point atomics: every
+// sum has a fixed order that depends on H and W only.
+constexpr int WCOLS = 32;    // columns per CTA of the column pass (one per lane)
+constexpr int WTILE = 32;    // square output tile of the Gaussian pass
+constexpr int WROWS = 64;    // image rows (one per thread) per CTA of the row pass
+
+struct WfmWs {
+  int* near;          // [B][H][W] nearest foreground row in the pixel's column, -1 if the column has none
+  int* stk_s;         // [B][H][W] per-row envelope stack: parabola (column) ...
+  int* stk_t;         // [B][H][W] ... and the first x it owns
+  unsigned char* etT; // [B][W][H] u8 prediction at the nearest foreground pixel, transposed
+  double* tab;        // [B][2][256] E for a background (0) / foreground (1) pixel of u8 value u
+  double* rowbg;      // [B][H] sum over the row's background pixels of E * (2 - 0.5^(D / 5))
+  double* tilefg;     // [B][tiles] sum over the tile's foreground pixels of min(E, EA)
+};
+
+static MetricWs carve_wfm(void* ws, int B, int H, int W, WfmWs* w, size_t* total) {
+  const size_t hw = (size_t)H * W, chunks = (size_t)cdiv(H, MROWS);
+  const size_t tiles = (size_t)cdiv(H, WTILE) * cdiv(W, WTILE);
+  size_t off = 0;
+  MetricWs m = {};
+  char* base = (char*)ws;
+  m.pu8 = (unsigned char*)(base + off); off = align256(off + B * hw);
+  m.gu8 = (unsigned char*)(base + off); off = align256(off + B * hw);
+  m.part1 = (long long*)(base + off); off = align256(off + B * chunks * NS1 * sizeof(long long));
+  m.info = (int*)(base + off); off = align256(off + (size_t)B * 4 * sizeof(int));
+  w->near = (int*)(base + off); off = align256(off + B * hw * sizeof(int));
+  w->stk_s = (int*)(base + off); off = align256(off + B * hw * sizeof(int));
+  w->stk_t = (int*)(base + off); off = align256(off + B * hw * sizeof(int));
+  w->etT = (unsigned char*)(base + off); off = align256(off + B * hw);
+  w->tab = (double*)(base + off); off = align256(off + (size_t)B * 512 * sizeof(double));
+  w->rowbg = (double*)(base + off); off = align256(off + (size_t)B * H * sizeof(double));
+  w->tilefg = (double*)(base + off); off = align256(off + B * tiles * sizeof(double));
+  if (total) *total = off;
+  return m;
+}
+
+// tab[b][g][u] = |p(u) - g| with p = (u/255 - min/255) / (max/255 - min/255) in the library's IEEE order
+__global__ void __launch_bounds__(256) wfm_table_kernel(MetricWs m, WfmWs w) {
+  const int b = blockIdx.x, u = threadIdx.x;
+  const int dmin = m.info[b * 4 + 0], R = m.info[b * 4 + 1];
+  const double p0 = __ddiv_rn((double)u, 255.0);
+  const double mn = __ddiv_rn((double)dmin, 255.0), mx = __ddiv_rn((double)(dmin + R), 255.0);
+  const double p = (dmin == 0 && R == 255) ? p0 : __ddiv_rn(__dsub_rn(p0, mn), __dsub_rn(mx, mn));
+  w.tab[b * 512 + u] = fabs(p);
+  w.tab[b * 512 + 256 + u] = fabs(__dsub_rn(p, 1.0));
+}
+
+// one lane per column, one warp per band of rows: band ends first, then each band scans down and up
+__global__ void __launch_bounds__(256) wfm_column_kernel(MetricWs m, WfmWs w, int H, int W) {
+  __shared__ int first[8][WCOLS], last[8][WCOLS];
+  const int b = blockIdx.y, lane = threadIdx.x & 31, band = threadIdx.x >> 5;
+  const int x = blockIdx.x * WCOLS + lane;
+  const int len = (H + 7) / 8, r0 = min(H, band * len), r1 = min(H, r0 + len);
+  const int64_t img = (int64_t)b * H * W;
+  const unsigned char* g = m.gu8 + img + x;
+  int* nr = w.near + img + x;
+  int f = -1, l = -1;
+  if (x < W)
+    for (int y = r0; y < r1; ++y)
+      if (g[(int64_t)y * W]) { if (f < 0) f = y; l = y; }
+  first[band][lane] = f;
+  last[band][lane] = l;
+  __syncthreads();
+  if (x >= W) return;
+  int up = -1, dn = -1;                      // nearest foreground row above the band / below it
+  for (int k = 0; k < band; ++k) if (last[k][lane] >= 0) up = last[k][lane];
+  for (int k = 7; k > band; --k) if (first[k][lane] >= 0) dn = first[k][lane];
+  for (int y = r1 - 1; y >= r0; --y) {       // nearest at or below y, parked in the output
+    if (g[(int64_t)y * W]) dn = y;
+    nr[(int64_t)y * W] = dn;
+  }
+  for (int y = r0; y < r1; ++y) {            // nearest at or above y; a tie goes to the lower row
+    if (g[(int64_t)y * W]) up = y;
+    const int d = nr[(int64_t)y * W];
+    nr[(int64_t)y * W] = (up >= 0 && (d < 0 || y - up <= d - y)) ? up : d;
+  }
+}
+
+// one thread per image row: lower envelope of f_j(x) = (x - j)^2 + (near_j - y)^2 over the columns j that have a
+// foreground pixel.  Parabola j gives way to u > j from x = sep(j, u) + 1 on, sep = floor((u^2 - j^2 + dy_u^2 -
+// dy_j^2) / (2 (u - j))): an x where both are equal stays with the lower column.
+__global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int B, int H, int W) {
+  const int64_t row = (int64_t)blockIdx.x * WROWS + threadIdx.x;
+  if (row >= (int64_t)B * H) return;
+  const int b = (int)(row / H), y = (int)(row - (int64_t)b * H);
+  const int64_t img = (int64_t)b * H * W;
+  const int* nr = w.near + row * W;
+  int* S = w.stk_s + row * W;
+  int* T = w.stk_t + row * W;
+  int q = -1, sq = 0, tq = 0;
+  long long dq2 = 0;                          // dy^2 of the top parabola
+  for (int u = 0; u < W; ++u) {
+    const int r = nr[u];
+    if (r < 0) continue;
+    const long long du2 = (long long)(r - y) * (r - y);
+    // pop while u is strictly below the top parabola where that one starts
+    while (q >= 0) {
+      const long long a = (long long)(tq - sq) * (tq - sq) + dq2, c = (long long)(tq - u) * (tq - u) + du2;
+      if (a <= c) break;
+      if (--q >= 0) {
+        sq = S[q]; tq = T[q];
+        const long long d = nr[sq] - y;
+        dq2 = d * d;
+      }
+    }
+    if (q < 0) {
+      q = 0; sq = u; tq = 0; dq2 = du2;
+      S[0] = u; T[0] = 0;
+    } else {
+      const long long num = (long long)u * u - (long long)sq * sq + du2 - dq2;     // >= 0 after the pops
+      const long long t = 1 + num / (2ll * (u - sq));
+      if (t < W) {
+        ++q; sq = u; tq = (int)t; dq2 = du2;
+        S[q] = u; T[q] = tq;
+      }
+    }
+  }
+  const unsigned char* pu = m.pu8 + img + (int64_t)y * W;
+  const unsigned char* gu = m.gu8 + img + (int64_t)y * W;
+  unsigned char* et = w.etT + img + y;
+  const double* tab0 = w.tab + b * 512;
+  constexpr double kLogHalfOver5 = -0.6931471805599453 / 5.0;    // np.log(0.5) / 5
+  double bg = 0.0;
+  if (q >= 0) {
+    int rq = nr[sq];
+    for (int x = W - 1; x >= 0; --x) {
+      et[(int64_t)x * H] = m.pu8[img + (int64_t)rq * W + sq];
+      if (!gu[x]) {
+        const long long dx = x - sq, dy = rq - y;
+        const double dist = sqrt((double)(dx * dx + dy * dy));
+        bg += __dmul_rn(tab0[pu[x]], __dsub_rn(2.0, exp(__dmul_rn(kLogHalfOver5, dist))));
+      }
+      if (x == tq && --q >= 0) { sq = S[q]; tq = T[q]; rq = nr[sq]; }
+    }
+  } else {                                    // no foreground in the image: the tail returns 0
+    for (int x = 0; x < W; ++x) et[(int64_t)x * H] = 0;
+  }
+  w.rowbg[row] = bg;
+}
+
+// matlab_style_gauss2D((7, 7), sigma = 5) as pysodmetrics evaluates it, indexed by (|dy|, |dx|)
+__constant__ double c_gauss7[4][4] = {
+    {0.023835778808354184, 0.023363798765182044, 0.022003197046847913, 0.019909316004406315},
+    {0.023363798765182044, 0.022901164553037447, 0.02156750455382744, 0.019515085133964022},
+    {0.022003197046847913, 0.02156750455382744, 0.02031151086671146, 0.018378615049044533},
+    {0.019909316004406315, 0.019515085133964022, 0.018378615049044533, 0.016629658588054284}};
+
+// EA = Et (*) K with zero padding at the foreground pixels of a 32 x 32 tile; sum of min(E, EA) over them
+__global__ void __launch_bounds__(256) wfm_gauss_kernel(MetricWs m, WfmWs w, int H, int W) {
+  constexpr int S = WTILE + 6;
+  __shared__ double et[S][S + 1];
+  __shared__ double red[256];
+  const int tiles_x = (W + WTILE - 1) / WTILE;
+  const int b = blockIdx.y, y0 = (blockIdx.x / tiles_x) * WTILE, x0 = (blockIdx.x % tiles_x) * WTILE;
+  const int64_t img = (int64_t)b * H * W;
+  const double* tab1 = w.tab + b * 512 + 256;
+  for (int i = threadIdx.x; i < S * S; i += 256) {      // lanes run along y: Et is stored transposed
+    const int yy = i % S, xx = i / S, y = y0 - 3 + yy, x = x0 - 3 + xx;
+    et[yy][xx] = (y >= 0 && y < H && x >= 0 && x < W) ? tab1[w.etT[img + (int64_t)x * H + y]] : 0.0;
+  }
+  __syncthreads();
+  const int tx = threadIdx.x & 31;
+  double s = 0.0;
+  for (int ty = threadIdx.x >> 5; ty < WTILE; ty += 8) {
+    const int y = y0 + ty, x = x0 + tx;
+    if (y >= H || x >= W || !m.gu8[img + (int64_t)y * W + x]) continue;
+    double ea = 0.0;
+#pragma unroll
+    for (int i = 0; i < 7; ++i)
+#pragma unroll
+      for (int j = 0; j < 7; ++j) ea = fma(c_gauss7[abs(i - 3)][abs(j - 3)], et[ty + i][tx + j], ea);
+    const double e = tab1[m.pu8[img + (int64_t)y * W + x]];
+    s += ea < e ? ea : e;
+  }
+  red[threadIdx.x] = s;
+  __syncthreads();
+  for (int o = 128; o > 0; o >>= 1) {
+    if (threadIdx.x < o) red[threadIdx.x] += red[threadIdx.x + o];
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) w.tilefg[(int64_t)b * gridDim.x + blockIdx.x] = red[0];
+}
+
+__global__ void wfm_final_kernel(MetricWs m, WfmWs w, int nchunks, int ntiles, int B, int H, double* __restrict__ out) {
+  const int b = blockIdx.x * blockDim.x + threadIdx.x;
+  if (b >= B) return;
+  long long n = 0;
+  for (int k = 0; k < nchunks; ++k) n += m.part1[((int64_t)b * nchunks + k) * NS1 + 2];
+  if (n == 0) { out[b] = 0.0; return; }
+  double fg = 0.0, bg = 0.0;
+  for (int k = 0; k < ntiles; ++k) fg += w.tilefg[(int64_t)b * ntiles + k];
+  for (int k = 0; k < H; ++k) bg += w.rowbg[(int64_t)b * H + k];
+  const double eps = 2.220446049250313e-16;
+  const double tpw = (double)n - fg;
+  const double R = 1.0 - fg / (double)n;
+  const double P = tpw / (tpw + bg + eps);
+  out[b] = 2.0 * R * P / (R + P + eps);
+}
+
 }  // namespace dgtd
 using namespace dgtd;
 
@@ -348,6 +557,40 @@ int dgtd_sod_metrics_fwd(const float* pred, const float* gt, void* ws, double* o
     metric_curves_kernel<<<B, 256, 0, s>>>(m, nchunks, H, W, curves);
     DGTD_LAUNCH_CHECK("sod_metrics(curves)");
   }
+  return 0;
+}
+
+int64_t dgtd_sod_wfm_ws_bytes(int B, int H, int W) {
+  if (B <= 0 || H <= 0 || W <= 0) return 0;
+  size_t total = 0;
+  WfmWs w;
+  carve_wfm(nullptr, B, H, W, &w, &total);
+  return (int64_t)total;
+}
+
+int dgtd_sod_wfm_fwd(const float* pred, const float* gt, void* ws, double* out, int B, int H, int W,
+                     dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(pred && gt && ws && out, "sod_wfm: null pointer");
+  DGTD_CHECK_ARG(B > 0 && H > 1 && W > 1 && (int64_t)H * W < (1ll << 28), "sod_wfm: bad shape");
+  DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_wfm: workspace must be 256-byte aligned");
+  cudaStream_t s = (cudaStream_t)stream;
+  WfmWs w;
+  MetricWs m = carve_wfm(ws, B, H, W, &w, nullptr);
+  const int nchunks = cdiv(H, MROWS), ntiles = cdiv(H, WTILE) * cdiv(W, WTILE);
+  metric_quantise_kernel<<<dim3(nchunks, B), 256, 0, s>>>(pred, gt, m, H, W);
+  DGTD_LAUNCH_CHECK("sod_wfm(quantise)");
+  metric_info_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, H, W);
+  DGTD_LAUNCH_CHECK("sod_wfm(info)");
+  wfm_table_kernel<<<B, 256, 0, s>>>(m, w);
+  DGTD_LAUNCH_CHECK("sod_wfm(table)");
+  wfm_column_kernel<<<dim3(cdiv(W, WCOLS), B), 256, 0, s>>>(m, w, H, W);
+  DGTD_LAUNCH_CHECK("sod_wfm(column)");
+  wfm_row_kernel<<<cdiv((int64_t)B * H, WROWS), WROWS, 0, s>>>(m, w, B, H, W);
+  DGTD_LAUNCH_CHECK("sod_wfm(row)");
+  wfm_gauss_kernel<<<dim3(ntiles, B), 256, 0, s>>>(m, w, H, W);
+  DGTD_LAUNCH_CHECK("sod_wfm(gauss)");
+  wfm_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, w, nchunks, ntiles, B, H, out);
+  DGTD_LAUNCH_CHECK("sod_wfm(final)");
   return 0;
 }
 

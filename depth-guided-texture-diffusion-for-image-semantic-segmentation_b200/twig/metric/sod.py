@@ -1,5 +1,6 @@
 """MAE, S-measure, F-measure and E-measure (twig/metric/{MAE,Smeasure,Fmeasure,Emeasure}.py:18-36: the four
-evaluators of config/cod.yml:123-128) computed by csrc/metric_ops.cu.
+evaluators of config/cod.yml:123-128) and the weighted F-measure of Margolin et al. (CVPR 2014) computed by
+csrc/metric_ops.cu.
 
 The reference moves prediction and label to the host and loops over images in numpy (pysodmetrics 1.3.1); here
 a batch is four kernel launches on the tensors `cod.forward(mode='predict')` returns, and 16 bytes per image come
@@ -16,15 +17,19 @@ import torch
 from ..ops import capi
 from ..ops.capi import call, check_cuda, ptr, stream
 
-__all__ = ["sod_metrics", "MAE", "Smeasure", "Fmeasure", "Emeasure"]
+__all__ = ["sod_metrics", "weighted_fmeasure", "MAE", "Smeasure", "Fmeasure", "Emeasure", "WeightedFmeasure"]
+
+
+def _check_maps(pred: torch.Tensor, gt: torch.Tensor) -> None:
+    check_cuda(pred, gt)
+    assert pred.dtype == torch.float32 and gt.dtype == torch.float32, "fp32 maps expected (cod.py:217)"
+    assert pred.shape == gt.shape and pred.dim() == 4 and pred.shape[1] == 1, (tuple(pred.shape), tuple(gt.shape))
 
 
 def sod_metrics(pred: torch.Tensor, gt: torch.Tensor, curves: bool = False):
     """pred, gt (B,1,H,W) fp32 in [0,1] on the GPU -> (B, 2) float64 = per-image (MAE, S-measure); with
     `curves=True` also (B, 2, 256) float64 = per-image changeable F-measure and E-measure curves."""
-    check_cuda(pred, gt)
-    assert pred.dtype == torch.float32 and gt.dtype == torch.float32, "fp32 maps expected (cod.py:217)"
-    assert pred.shape == gt.shape and pred.dim() == 4 and pred.shape[1] == 1, (tuple(pred.shape), tuple(gt.shape))
+    _check_maps(pred, gt)
     B, _, H, W = pred.shape
     ws = torch.empty(int(capi.load().dgtd_sod_metrics_ws_bytes(B, H, W)), device=pred.device, dtype=torch.uint8)
     out = torch.empty(B, 2, device=pred.device, dtype=torch.float64)
@@ -33,9 +38,26 @@ def sod_metrics(pred: torch.Tensor, gt: torch.Tensor, curves: bool = False):
     return (out, cur) if curves else out
 
 
+def weighted_fmeasure(pred: torch.Tensor, gt: torch.Tensor) -> torch.Tensor:
+    """pred, gt (B,1,H,W) fp32 in [0,1] on the GPU -> (B,) float64 = per-image weighted F-measure (pysodmetrics
+    `WeightedFmeasure`, beta = 1; 0 for an empty ground truth).  H and W must both exceed 1."""
+    _check_maps(pred, gt)
+    B, _, H, W = pred.shape
+    ws = torch.empty(int(capi.load().dgtd_sod_wfm_ws_bytes(B, H, W)), device=pred.device, dtype=torch.uint8)
+    out = torch.empty(B, device=pred.device, dtype=torch.float64)
+    call("dgtd_sod_wfm_fwd", ptr(pred), ptr(gt), ptr(ws), ptr(out), B, H, W, stream())
+    return out
+
+
+def _sod_column(column: int):
+    return lambda pred, gt: sod_metrics(pred, gt)[:, column]
+
+
 class _Running:
+    """The evaluator keeps every image's value; a batch records the mean over all images seen so far.  `_per_image`
+    maps a (pred, gt) batch to its (B,) values."""
     default_prefix = 'COD'
-    _column = 0
+    _per_image = None
     _key = ''
     _name = ''
 
@@ -48,7 +70,7 @@ class _Running:
 
     def process(self, data_batch, data_samples: Tuple[torch.Tensor, torch.Tensor]) -> None:
         pred, gt = data_samples
-        vals = sod_metrics(pred.detach().float().contiguous(), gt.detach().float().contiguous())[:, self._column]
+        vals = self._per_image(pred.detach().float().contiguous(), gt.detach().float().contiguous())
         for v in vals.cpu().tolist():           # the evaluator's list of per-image values, as a running sum
             self._sum += v
             self._count += 1
@@ -103,9 +125,14 @@ class Emeasure(_RunningCurve):
 
 class MAE(_Running):
     """twig/metric/MAE.py."""
-    _column, _key, _name = 0, 'mae', 'MAE'
+    _per_image, _key, _name = staticmethod(_sod_column(0)), 'mae', 'MAE'
 
 
 class Smeasure(_Running):
     """twig/metric/Smeasure.py."""
-    _column, _key, _name = 1, 'sm', 'Smeasure'
+    _per_image, _key, _name = staticmethod(_sod_column(1)), 'sm', 'Smeasure'
+
+
+class WeightedFmeasure(_Running):
+    """twig/metric/WeightedFmeasure.py (commented out in the reference): pysodmetrics `WeightedFmeasure`."""
+    _per_image, _key, _name = staticmethod(weighted_fmeasure), 'wfm', 'WeightedFmeasure'

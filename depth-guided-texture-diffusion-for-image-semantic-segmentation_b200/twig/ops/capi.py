@@ -131,8 +131,11 @@ SIGNATURES = {
     "dgtd_adamw_step": [_P, _P, _P, _P, _P, _I, _F, _F, _F, _I, _F, _F, _P],
     "dgtd_sod_metrics_ws_bytes": [_I, _I, _I],
     "dgtd_sod_metrics_fwd": [_P, _P, _P, _P, _P, _I, _I, _I, _P],
+    "dgtd_sod_wfm_ws_bytes": [_I, _I, _I],
+    "dgtd_sod_wfm_fwd": [_P, _P, _P, _P, _I, _I, _I, _P],
 }
 _RESTYPES = {"dgtd_last_error": c_char_p, "dgtd_launch_count": c_int64, "dgtd_sod_metrics_ws_bytes": c_int64,
+             "dgtd_sod_wfm_ws_bytes": c_int64,
              "dgtd_col_stats_ws_bytes": c_int64, "dgtd_attention_bwd_ws_floats": c_int64, "dgtd_dwconv3_gelu_bwd_ws_floats": c_int64, "dgtd_gate_bwd_ws_floats": c_int64, "dgtd_prelu_bwd_ws_bytes": c_int64}
 
 _lib: Optional[ctypes.CDLL] = None

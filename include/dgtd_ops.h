@@ -492,6 +492,15 @@ int dgtd_resize_nhwc_ld_bwd(const float* g, int ldg, float* dx, int lddx, int B,
 int64_t dgtd_sod_metrics_ws_bytes(int B, int H, int W);
 int dgtd_sod_metrics_fwd(const float* pred, const float* gt, void* ws, double* out, double* curves, int B, int H,
                          int W, dgtd_stream_t stream);
+/* weighted F-measure (Margolin et al., CVPR 2014; pysodmetrics 1.3.1 `WeightedFmeasure`, beta = 1): same inputs,
+ * quantisation and normalisation as dgtd_sod_metrics_fwd; out[b] = F^w of image b in float64 (0 for an empty ground
+ * truth).  Every background pixel takes the error of its nearest foreground pixel under the exact Euclidean distance;
+ * among equidistant ones the pixel with the lowest column, then the lowest row, is taken (the choice of
+ * scipy.ndimage.distance_transform_edt(return_indices=True)).  Fixed-order reductions: bit-stable, independent of
+ * batch composition.  H > 1, W > 1, H * W < 2^28.  ws: 256-byte aligned scratch of dgtd_sod_wfm_ws_bytes(B, H, W). */
+int64_t dgtd_sod_wfm_ws_bytes(int B, int H, int W);
+int dgtd_sod_wfm_fwd(const float* pred, const float* gt, void* ws, double* out, int B, int H, int W,
+                     dgtd_stream_t stream);
 
 /* ---- optimizer step of the training configuration (config/sod.yml:56-76; torch.optim.AdamW semantics) ----------
  * One launch over flat fp32 buffers p, g, m, v (the hot path's gradients already live in one flat buffer,
