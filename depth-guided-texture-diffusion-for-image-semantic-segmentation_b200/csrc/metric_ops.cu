@@ -8,6 +8,8 @@
 // float64 from the exact integers (variances as N*S2 - S1^2: no cancellation).  No atomics, no floating-point
 // reduction: results are bit-stable and independent of the launch geometry.  The weighted F-measure (below
 // metric_curves_kernel) reuses the quantise and info passes and adds an exact Euclidean distance transform.
+#include <math_constants.h>
+
 #include "common.cuh"
 
 namespace dgtd {
@@ -42,6 +44,35 @@ static MetricWs carve(void* ws, int B, int H, int W, size_t* total) {
   return m;
 }
 
+// Per-image geometry.  Every image owns an H x W slot (row pitch W) of the batch tensors and of the workspace.
+// `Dense`: the image fills its slot.  `Sized`: image b is the top-left sizes[b] = (H_b, W_b) of its slot and the rest
+// of the slot is never read; a size outside [2, H] x [2, W] reads as 0 x 0, so the image does no work and its outputs
+// are NaN.  Chunks, rows and tiles of the slot outside the image write identity partials, so an image's values equal
+// a Dense call on its crop alone, bit for bit.
+struct Dims { int h, w; };
+
+struct Dense {
+  static constexpr bool sized = false;
+  int H, W;
+  __device__ __forceinline__ Dims dims(int) const { return {H, W}; }
+  // slot offset of pixel i (row-major index within an image of width w)
+  __device__ __forceinline__ int64_t at(int i, int) const { return i; }
+};
+
+struct Sized {
+  static constexpr bool sized = true;
+  const int* sizes;   // [B][2] = (H_b, W_b)
+  int H, W;
+  __device__ __forceinline__ Dims dims(int b) const {
+    const int h = sizes[2 * b], w = sizes[2 * b + 1];
+    return (h >= 2 && h <= H && w >= 2 && w <= W) ? Dims{h, w} : Dims{0, 0};
+  }
+  __device__ __forceinline__ int64_t at(int i, int w) const {
+    const int r = i / w;
+    return (int64_t)r * W + (i - r * w);
+  }
+};
+
 __device__ __forceinline__ long long warp_sum_ll(long long v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v += __shfl_xor_sync(0xffffffffu, v, o);
@@ -49,21 +80,25 @@ __device__ __forceinline__ long long warp_sum_ll(long long v) {
 }
 
 // pass 1: `(x * 255).astype(np.uint8)` (Smeasure.py:25-26), gt > 128, per-band statistics
+template <class G>
 __global__ void __launch_bounds__(256) metric_quantise_kernel(const float* __restrict__ pred, const float* __restrict__ gt,
-                                                              MetricWs m, int H, int W) {
+                                                              MetricWs m, G geo) {
   __shared__ long long red[8][NS1];
   const int b = blockIdx.y, chunk = blockIdx.x, nchunks = gridDim.x;
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w;
   const int r0 = chunk * MROWS, r1 = min(H, r0 + MROWS);
-  const int64_t img = (int64_t)b * H * W;
+  const int64_t img = (int64_t)b * geo.H * geo.W;
   int vmin = 255, vmax = 0;
   long long cnt = 0, srow = 0, scol = 0;
   for (int i = r0 * W + threadIdx.x; i < r1 * W; i += 256) {
-    const float p = pred[img + i], g = gt[img + i];
+    const int64_t o = img + geo.at(i, W);
+    const float p = pred[o], g = gt[o];
     const int pu = (int)(unsigned char)(int)(__fmul_rn(p, 255.0f));     // truncation toward zero, like astype
     const int gu = (int)(unsigned char)(int)(__fmul_rn(g, 255.0f));
     const int fg = gu > 128;
-    m.pu8[img + i] = (unsigned char)pu;
-    m.gu8[img + i] = (unsigned char)fg;
+    m.pu8[o] = (unsigned char)pu;
+    m.gu8[o] = (unsigned char)fg;
     vmin = min(vmin, pu);
     vmax = max(vmax, pu);
     if (fg) {
@@ -97,9 +132,11 @@ __global__ void __launch_bounds__(256) metric_quantise_kernel(const float* __res
 }
 
 // per image: min-max normalisation constants (`_prepare_data`) and the centroid split (`Smeasure.centroid`)
-__global__ void metric_info_kernel(MetricWs m, int nchunks, int B, int H, int W) {
+template <class G>
+__global__ void metric_info_kernel(MetricWs m, int nchunks, int B, G geo) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const Dims d = geo.dims(b);
   const long long* p = m.part1 + (int64_t)b * nchunks * NS1;
   long long a = 255, c = 0, n = 0, sr = 0, sc = 0;
   for (int k = 0; k < nchunks; ++k) {
@@ -109,7 +146,7 @@ __global__ void metric_info_kernel(MetricWs m, int nchunks, int B, int H, int W)
   if (R == 0) { dmin = 0; R = 255; }          // constant prediction: pred / 255 is left un-normalised
   double x, y;
   if (n == 0) {
-    x = rint((double)W / 2.0); y = rint((double)H / 2.0);     // np.round = half to even
+    x = rint((double)d.w / 2.0); y = rint((double)d.h / 2.0);     // np.round = half to even
   } else {
     y = rint((double)sr / (double)n); x = rint((double)sc / (double)n);
   }
@@ -118,17 +155,21 @@ __global__ void metric_info_kernel(MetricWs m, int nchunks, int B, int H, int W)
 }
 
 // pass 2: integer moments per centroid quadrant
-__global__ void __launch_bounds__(256) metric_moments_kernel(MetricWs m, int H, int W) {
+template <class G>
+__global__ void __launch_bounds__(256) metric_moments_kernel(MetricWs m, G geo) {
   __shared__ unsigned long long red[8][NS2];
   const int b = blockIdx.y, chunk = blockIdx.x, nchunks = gridDim.x;
+  const Dims dm = geo.dims(b);
+  const int H = dm.h, W = dm.w;
   const int r0 = chunk * MROWS, r1 = min(H, r0 + MROWS);
-  const int64_t img = (int64_t)b * H * W;
+  const int64_t img = (int64_t)b * geo.H * geo.W;
   const int dmin = m.info[b * 4 + 0], cx = m.info[b * 4 + 2], cy = m.info[b * 4 + 3];
   unsigned int s[NS2];
 #pragma unroll
   for (int k = 0; k < NS2; ++k) s[k] = 0u;
   for (int i = r0 * W + threadIdx.x; i < r1 * W; i += 256) {
-    const unsigned int d = (unsigned int)((int)m.pu8[img + i] - dmin), g = m.gu8[img + i];
+    const int64_t o = img + geo.at(i, W);
+    const unsigned int d = (unsigned int)((int)m.pu8[o] - dmin), g = m.gu8[o];
     const int r = i / W, c = i - r * W;
     const int q = (r >= cy ? 2 : 0) + (c >= cx ? 1 : 0);
 #pragma unroll
@@ -178,9 +219,13 @@ __device__ double s_object_from_moments(double n, double S1, double S2, double R
   return 2.0 * x / (x * x + 1.0 + sigma + 2.220446049250313e-16);
 }
 
-__global__ void metric_final_kernel(MetricWs m, int nchunks, int B, int H, int W, double* __restrict__ out) {
+template <class G>
+__global__ void metric_final_kernel(MetricWs m, int nchunks, int B, G geo, double* __restrict__ out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w;
+  if (G::sized && H == 0) { out[b * 2 + 0] = out[b * 2 + 1] = CUDART_NAN; return; }
   double S[NS2];
   for (int k = 0; k < NS2; ++k) {
     unsigned long long v = 0;
@@ -232,7 +277,8 @@ __global__ void metric_final_kernel(MetricWs m, int nchunks, int B, int H, int W
 // does that re-quantisation in float64 -- (u/255 - min/255) / (max/255 - min/255) * 255, truncated -- and a value
 // that lands on an integer can fall either side of it, so the 256-entry map is evaluated with the same IEEE
 // operations in the same order (explicit round-to-nearest intrinsics: no contraction).
-__global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, int H, int W) {
+template <class G>
+__global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, G geo) {
   __shared__ unsigned int hist[512];
   __shared__ unsigned char lut[256];
   const int b = blockIdx.y, chunk = blockIdx.x, nchunks = gridDim.x;
@@ -250,10 +296,14 @@ __global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, int H, int
     hist[256 + u] = 0u;
   }
   __syncthreads();
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w;
   const int r0 = chunk * MROWS, r1 = min(H, r0 + MROWS);
-  const int64_t img = (int64_t)b * H * W;
-  for (int i = r0 * W + threadIdx.x; i < r1 * W; i += 256)
-    atomicAdd(&hist[(m.gu8[img + i] ? 0 : 256) + lut[m.pu8[img + i]]], 1u);   // integer: exact in any order
+  const int64_t img = (int64_t)b * geo.H * geo.W;
+  for (int i = r0 * W + threadIdx.x; i < r1 * W; i += 256) {
+    const int64_t o = img + geo.at(i, W);
+    atomicAdd(&hist[(m.gu8[o] ? 0 : 256) + lut[m.pu8[o]]], 1u);   // integer: exact in any order
+  }
   __syncthreads();
   unsigned int* o = m.part3 + ((int64_t)b * nchunks + chunk) * 512;
   o[threadIdx.x] = hist[threadIdx.x];
@@ -261,9 +311,15 @@ __global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, int H, int
 }
 
 // curves[b][0][i] = changeable F-measure, curves[b][1][i] = E-measure at threshold 255 - i (the library's order)
-__global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchunks, int H, int W, double* __restrict__ curves) {
+template <class G>
+__global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchunks, G geo, double* __restrict__ curves) {
   __shared__ double cf[256], cb[256];
   const int b = blockIdx.x, t = threadIdx.x;
+  const Dims d = geo.dims(b);
+  if (G::sized && d.h == 0) {
+    curves[((int64_t)b * 2 + 0) * 256 + t] = curves[((int64_t)b * 2 + 1) * 256 + t] = CUDART_NAN;
+    return;
+  }
   unsigned long long f = 0, g = 0;
   for (int c = 0; c < nchunks; ++c) {
     const unsigned int* o = m.part3 + ((int64_t)b * nchunks + c) * 512;
@@ -278,7 +334,7 @@ __global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchu
   }
   __syncthreads();
   const double eps = 2.220446049250313e-16;
-  const double size = (double)H * (double)W, gt_fg = cf[255];
+  const double size = (double)d.h * (double)d.w, gt_fg = cf[255];
   const double fg_fg = cf[t], fg_bg = cb[t];
   // Fmeasure.cal_pr, beta^2 = 0.3
   {
@@ -329,6 +385,8 @@ constexpr int WCOLS = 32;    // columns per CTA of the column pass (one per lane
 constexpr int WTILE = 32;    // square output tile of the Gaussian pass
 constexpr int WROWS = 64;    // image rows (one per thread) per CTA of the row pass
 
+__device__ __forceinline__ int cdiv_d(int a, int b) { return (a + b - 1) / b; }
+
 struct WfmWs {
   int* near;          // [B][H][W] nearest foreground row in the pixel's column, -1 if the column has none
   int* stk_s;         // [B][H][W] per-row envelope stack: parabola (column) ...
@@ -372,18 +430,21 @@ __global__ void __launch_bounds__(256) wfm_table_kernel(MetricWs m, WfmWs w) {
 }
 
 // one lane per column, one warp per band of rows: band ends first, then each band scans down and up
-__global__ void __launch_bounds__(256) wfm_column_kernel(MetricWs m, WfmWs w, int H, int W) {
+template <class G>
+__global__ void __launch_bounds__(256) wfm_column_kernel(MetricWs m, WfmWs w, G geo) {
   __shared__ int first[8][WCOLS], last[8][WCOLS];
   const int b = blockIdx.y, lane = threadIdx.x & 31, band = threadIdx.x >> 5;
   const int x = blockIdx.x * WCOLS + lane;
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w, P = geo.W;
   const int len = (H + 7) / 8, r0 = min(H, band * len), r1 = min(H, r0 + len);
-  const int64_t img = (int64_t)b * H * W;
+  const int64_t img = (int64_t)b * geo.H * geo.W;
   const unsigned char* g = m.gu8 + img + x;
   int* nr = w.near + img + x;
   int f = -1, l = -1;
   if (x < W)
     for (int y = r0; y < r1; ++y)
-      if (g[(int64_t)y * W]) { if (f < 0) f = y; l = y; }
+      if (g[(int64_t)y * P]) { if (f < 0) f = y; l = y; }
   first[band][lane] = f;
   last[band][lane] = l;
   __syncthreads();
@@ -392,27 +453,31 @@ __global__ void __launch_bounds__(256) wfm_column_kernel(MetricWs m, WfmWs w, in
   for (int k = 0; k < band; ++k) if (last[k][lane] >= 0) up = last[k][lane];
   for (int k = 7; k > band; --k) if (first[k][lane] >= 0) dn = first[k][lane];
   for (int y = r1 - 1; y >= r0; --y) {       // nearest at or below y, parked in the output
-    if (g[(int64_t)y * W]) dn = y;
-    nr[(int64_t)y * W] = dn;
+    if (g[(int64_t)y * P]) dn = y;
+    nr[(int64_t)y * P] = dn;
   }
   for (int y = r0; y < r1; ++y) {            // nearest at or above y; a tie goes to the lower row
-    if (g[(int64_t)y * W]) up = y;
-    const int d = nr[(int64_t)y * W];
-    nr[(int64_t)y * W] = (up >= 0 && (d < 0 || y - up <= d - y)) ? up : d;
+    if (g[(int64_t)y * P]) up = y;
+    const int d = nr[(int64_t)y * P];
+    nr[(int64_t)y * P] = (up >= 0 && (d < 0 || y - up <= d - y)) ? up : d;
   }
 }
 
 // one thread per image row: lower envelope of f_j(x) = (x - j)^2 + (near_j - y)^2 over the columns j that have a
 // foreground pixel.  Parabola j gives way to u > j from x = sep(j, u) + 1 on, sep = floor((u^2 - j^2 + dy_u^2 -
 // dy_j^2) / (2 (u - j))): an x where both are equal stays with the lower column.
-__global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int B, int H, int W) {
+template <class G>
+__global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int B, G geo) {
   const int64_t row = (int64_t)blockIdx.x * WROWS + threadIdx.x;
-  if (row >= (int64_t)B * H) return;
-  const int b = (int)(row / H), y = (int)(row - (int64_t)b * H);
-  const int64_t img = (int64_t)b * H * W;
-  const int* nr = w.near + row * W;
-  int* S = w.stk_s + row * W;
-  int* T = w.stk_t + row * W;
+  if (row >= (int64_t)B * geo.H) return;
+  const int b = (int)(row / geo.H), y = (int)(row - (int64_t)b * geo.H);
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w, P = geo.W, PT = geo.H;
+  if (G::sized && y >= H) return;            // below the image: the tail does not read rowbg[y]
+  const int64_t img = (int64_t)b * geo.H * geo.W;
+  const int* nr = w.near + row * P;
+  int* S = w.stk_s + row * P;
+  int* T = w.stk_t + row * P;
   int q = -1, sq = 0, tq = 0;
   long long dq2 = 0;                          // dy^2 of the top parabola
   for (int u = 0; u < W; ++u) {
@@ -441,8 +506,8 @@ __global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int
       }
     }
   }
-  const unsigned char* pu = m.pu8 + img + (int64_t)y * W;
-  const unsigned char* gu = m.gu8 + img + (int64_t)y * W;
+  const unsigned char* pu = m.pu8 + img + (int64_t)y * P;
+  const unsigned char* gu = m.gu8 + img + (int64_t)y * P;
   unsigned char* et = w.etT + img + y;
   const double* tab0 = w.tab + b * 512;
   constexpr double kLogHalfOver5 = -0.6931471805599453 / 5.0;    // np.log(0.5) / 5
@@ -450,7 +515,7 @@ __global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int
   if (q >= 0) {
     int rq = nr[sq];
     for (int x = W - 1; x >= 0; --x) {
-      et[(int64_t)x * H] = m.pu8[img + (int64_t)rq * W + sq];
+      et[(int64_t)x * PT] = m.pu8[img + (int64_t)rq * P + sq];
       if (!gu[x]) {
         const long long dx = x - sq, dy = rq - y;
         const double dist = sqrt((double)(dx * dx + dy * dy));
@@ -459,7 +524,7 @@ __global__ void __launch_bounds__(WROWS) wfm_row_kernel(MetricWs m, WfmWs w, int
       if (x == tq && --q >= 0) { sq = S[q]; tq = T[q]; rq = nr[sq]; }
     }
   } else {                                    // no foreground in the image: the tail returns 0
-    for (int x = 0; x < W; ++x) et[(int64_t)x * H] = 0;
+    for (int x = 0; x < W; ++x) et[(int64_t)x * PT] = 0;
   }
   w.rowbg[row] = bg;
 }
@@ -472,30 +537,37 @@ __constant__ double c_gauss7[4][4] = {
     {0.019909316004406315, 0.019515085133964022, 0.018378615049044533, 0.016629658588054284}};
 
 // EA = Et (*) K with zero padding at the foreground pixels of a 32 x 32 tile; sum of min(E, EA) over them
-__global__ void __launch_bounds__(256) wfm_gauss_kernel(MetricWs m, WfmWs w, int H, int W) {
+template <class G>
+__global__ void __launch_bounds__(256) wfm_gauss_kernel(MetricWs m, WfmWs w, G geo) {
   constexpr int S = WTILE + 6;
   __shared__ double et[S][S + 1];
   __shared__ double red[256];
-  const int tiles_x = (W + WTILE - 1) / WTILE;
+  const int tiles_x = (geo.W + WTILE - 1) / WTILE;
   const int b = blockIdx.y, y0 = (blockIdx.x / tiles_x) * WTILE, x0 = (blockIdx.x % tiles_x) * WTILE;
-  const int64_t img = (int64_t)b * H * W;
+  const Dims d = geo.dims(b);
+  const int H = d.h, W = d.w, P = geo.W, PT = geo.H;
+  if (G::sized && (y0 >= H || x0 >= W)) {                // outside the image: the tail does not read it
+    if (threadIdx.x == 0) w.tilefg[(int64_t)b * gridDim.x + blockIdx.x] = 0.0;
+    return;
+  }
+  const int64_t img = (int64_t)b * geo.H * geo.W;
   const double* tab1 = w.tab + b * 512 + 256;
   for (int i = threadIdx.x; i < S * S; i += 256) {      // lanes run along y: Et is stored transposed
     const int yy = i % S, xx = i / S, y = y0 - 3 + yy, x = x0 - 3 + xx;
-    et[yy][xx] = (y >= 0 && y < H && x >= 0 && x < W) ? tab1[w.etT[img + (int64_t)x * H + y]] : 0.0;
+    et[yy][xx] = (y >= 0 && y < H && x >= 0 && x < W) ? tab1[w.etT[img + (int64_t)x * PT + y]] : 0.0;
   }
   __syncthreads();
   const int tx = threadIdx.x & 31;
   double s = 0.0;
   for (int ty = threadIdx.x >> 5; ty < WTILE; ty += 8) {
     const int y = y0 + ty, x = x0 + tx;
-    if (y >= H || x >= W || !m.gu8[img + (int64_t)y * W + x]) continue;
+    if (y >= H || x >= W || !m.gu8[img + (int64_t)y * P + x]) continue;
     double ea = 0.0;
 #pragma unroll
     for (int i = 0; i < 7; ++i)
 #pragma unroll
       for (int j = 0; j < 7; ++j) ea = fma(c_gauss7[abs(i - 3)][abs(j - 3)], et[ty + i][tx + j], ea);
-    const double e = tab1[m.pu8[img + (int64_t)y * W + x]];
+    const double e = tab1[m.pu8[img + (int64_t)y * P + x]];
     s += ea < e ? ea : e;
   }
   red[threadIdx.x] = s;
@@ -507,20 +579,72 @@ __global__ void __launch_bounds__(256) wfm_gauss_kernel(MetricWs m, WfmWs w, int
   if (threadIdx.x == 0) w.tilefg[(int64_t)b * gridDim.x + blockIdx.x] = red[0];
 }
 
-__global__ void wfm_final_kernel(MetricWs m, WfmWs w, int nchunks, int ntiles, int B, int H, double* __restrict__ out) {
+// The image's own rows and its own cdiv(H_b, 32) x cdiv(W_b, 32) tiles, in row-major order: the float64 sums of a
+// Sized call run in the order of a Dense call on the crop.
+template <class G>
+__global__ void wfm_final_kernel(MetricWs m, WfmWs w, int nchunks, int ntiles, int B, G geo, double* __restrict__ out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
+  const Dims d = geo.dims(b);
+  if (G::sized && d.h == 0) { out[b] = CUDART_NAN; return; }
   long long n = 0;
   for (int k = 0; k < nchunks; ++k) n += m.part1[((int64_t)b * nchunks + k) * NS1 + 2];
   if (n == 0) { out[b] = 0.0; return; }
   double fg = 0.0, bg = 0.0;
-  for (int k = 0; k < ntiles; ++k) fg += w.tilefg[(int64_t)b * ntiles + k];
-  for (int k = 0; k < H; ++k) bg += w.rowbg[(int64_t)b * H + k];
+  const int tiles_x = cdiv_d(geo.W, WTILE), ty1 = cdiv_d(d.h, WTILE), tx1 = cdiv_d(d.w, WTILE);
+  for (int ty = 0; ty < ty1; ++ty)
+    for (int tx = 0; tx < tx1; ++tx) fg += w.tilefg[(int64_t)b * ntiles + ty * tiles_x + tx];
+  for (int k = 0; k < d.h; ++k) bg += w.rowbg[(int64_t)b * geo.H + k];
   const double eps = 2.220446049250313e-16;
   const double tpw = (double)n - fg;
   const double R = 1.0 - fg / (double)n;
   const double P = tpw / (tpw + bg + eps);
   out[b] = 2.0 * R * P / (R + P + eps);
+}
+
+template <class G>
+static int launch_sod_metrics(const float* pred, const float* gt, void* ws, double* out, double* curves, int B, G geo,
+                              cudaStream_t s) {
+  MetricWs m = carve(ws, B, geo.H, geo.W, nullptr);
+  const int nchunks = cdiv(geo.H, MROWS);
+  metric_quantise_kernel<<<dim3(nchunks, B), 256, 0, s>>>(pred, gt, m, geo);
+  DGTD_LAUNCH_CHECK("sod_metrics(quantise)");
+  metric_info_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, geo);
+  DGTD_LAUNCH_CHECK("sod_metrics(info)");
+  metric_moments_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, geo);
+  DGTD_LAUNCH_CHECK("sod_metrics(moments)");
+  metric_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, geo, out);
+  DGTD_LAUNCH_CHECK("sod_metrics(final)");
+  if (curves) {
+    metric_hist_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, geo);
+    DGTD_LAUNCH_CHECK("sod_metrics(hist)");
+    metric_curves_kernel<<<B, 256, 0, s>>>(m, nchunks, geo, curves);
+    DGTD_LAUNCH_CHECK("sod_metrics(curves)");
+  }
+  return 0;
+}
+
+template <class G>
+static int launch_sod_wfm(const float* pred, const float* gt, void* ws, double* out, int B, G geo, cudaStream_t s) {
+  const int H = geo.H, W = geo.W;
+  WfmWs w;
+  MetricWs m = carve_wfm(ws, B, H, W, &w, nullptr);
+  const int nchunks = cdiv(H, MROWS), ntiles = cdiv(H, WTILE) * cdiv(W, WTILE);
+  metric_quantise_kernel<<<dim3(nchunks, B), 256, 0, s>>>(pred, gt, m, geo);
+  DGTD_LAUNCH_CHECK("sod_wfm(quantise)");
+  metric_info_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, geo);
+  DGTD_LAUNCH_CHECK("sod_wfm(info)");
+  wfm_table_kernel<<<B, 256, 0, s>>>(m, w);
+  DGTD_LAUNCH_CHECK("sod_wfm(table)");
+  wfm_column_kernel<<<dim3(cdiv(W, WCOLS), B), 256, 0, s>>>(m, w, geo);
+  DGTD_LAUNCH_CHECK("sod_wfm(column)");
+  wfm_row_kernel<<<cdiv((int64_t)B * H, WROWS), WROWS, 0, s>>>(m, w, B, geo);
+  DGTD_LAUNCH_CHECK("sod_wfm(row)");
+  wfm_gauss_kernel<<<dim3(ntiles, B), 256, 0, s>>>(m, w, geo);
+  DGTD_LAUNCH_CHECK("sod_wfm(gauss)");
+  wfm_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, w, nchunks, ntiles, B, geo, out);
+  DGTD_LAUNCH_CHECK("sod_wfm(final)");
+  return 0;
 }
 
 }  // namespace dgtd
@@ -540,24 +664,15 @@ int dgtd_sod_metrics_fwd(const float* pred, const float* gt, void* ws, double* o
   DGTD_CHECK_ARG(pred && gt && ws && out, "sod_metrics: null pointer");
   DGTD_CHECK_ARG(B > 0 && H > 1 && W > 1 && (int64_t)H * W < (1ll << 28), "sod_metrics: bad shape");
   DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics: workspace must be 256-byte aligned");
-  cudaStream_t s = (cudaStream_t)stream;
-  MetricWs m = carve(ws, B, H, W, nullptr);
-  const int nchunks = cdiv(H, MROWS);
-  metric_quantise_kernel<<<dim3(nchunks, B), 256, 0, s>>>(pred, gt, m, H, W);
-  DGTD_LAUNCH_CHECK("sod_metrics(quantise)");
-  metric_info_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, H, W);
-  DGTD_LAUNCH_CHECK("sod_metrics(info)");
-  metric_moments_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, H, W);
-  DGTD_LAUNCH_CHECK("sod_metrics(moments)");
-  metric_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, H, W, out);
-  DGTD_LAUNCH_CHECK("sod_metrics(final)");
-  if (curves) {
-    metric_hist_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, H, W);
-    DGTD_LAUNCH_CHECK("sod_metrics(hist)");
-    metric_curves_kernel<<<B, 256, 0, s>>>(m, nchunks, H, W, curves);
-    DGTD_LAUNCH_CHECK("sod_metrics(curves)");
-  }
-  return 0;
+  return launch_sod_metrics(pred, gt, ws, out, curves, B, Dense{H, W}, (cudaStream_t)stream);
+}
+
+int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out,
+                               double* curves, int B, int Hmax, int Wmax, dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(pred && gt && sizes && ws && out, "sod_metrics: null pointer");
+  DGTD_CHECK_ARG(B > 0 && Hmax > 1 && Wmax > 1 && (int64_t)Hmax * Wmax < (1ll << 28), "sod_metrics: bad shape");
+  DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics: workspace must be 256-byte aligned");
+  return launch_sod_metrics(pred, gt, ws, out, curves, B, Sized{sizes, Hmax, Wmax}, (cudaStream_t)stream);
 }
 
 int64_t dgtd_sod_wfm_ws_bytes(int B, int H, int W) {
@@ -573,25 +688,15 @@ int dgtd_sod_wfm_fwd(const float* pred, const float* gt, void* ws, double* out, 
   DGTD_CHECK_ARG(pred && gt && ws && out, "sod_wfm: null pointer");
   DGTD_CHECK_ARG(B > 0 && H > 1 && W > 1 && (int64_t)H * W < (1ll << 28), "sod_wfm: bad shape");
   DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_wfm: workspace must be 256-byte aligned");
-  cudaStream_t s = (cudaStream_t)stream;
-  WfmWs w;
-  MetricWs m = carve_wfm(ws, B, H, W, &w, nullptr);
-  const int nchunks = cdiv(H, MROWS), ntiles = cdiv(H, WTILE) * cdiv(W, WTILE);
-  metric_quantise_kernel<<<dim3(nchunks, B), 256, 0, s>>>(pred, gt, m, H, W);
-  DGTD_LAUNCH_CHECK("sod_wfm(quantise)");
-  metric_info_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, H, W);
-  DGTD_LAUNCH_CHECK("sod_wfm(info)");
-  wfm_table_kernel<<<B, 256, 0, s>>>(m, w);
-  DGTD_LAUNCH_CHECK("sod_wfm(table)");
-  wfm_column_kernel<<<dim3(cdiv(W, WCOLS), B), 256, 0, s>>>(m, w, H, W);
-  DGTD_LAUNCH_CHECK("sod_wfm(column)");
-  wfm_row_kernel<<<cdiv((int64_t)B * H, WROWS), WROWS, 0, s>>>(m, w, B, H, W);
-  DGTD_LAUNCH_CHECK("sod_wfm(row)");
-  wfm_gauss_kernel<<<dim3(ntiles, B), 256, 0, s>>>(m, w, H, W);
-  DGTD_LAUNCH_CHECK("sod_wfm(gauss)");
-  wfm_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, w, nchunks, ntiles, B, H, out);
-  DGTD_LAUNCH_CHECK("sod_wfm(final)");
-  return 0;
+  return launch_sod_wfm(pred, gt, ws, out, B, Dense{H, W}, (cudaStream_t)stream);
+}
+
+int dgtd_sod_wfm_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out, int B,
+                           int Hmax, int Wmax, dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(pred && gt && sizes && ws && out, "sod_wfm: null pointer");
+  DGTD_CHECK_ARG(B > 0 && Hmax > 1 && Wmax > 1 && (int64_t)Hmax * Wmax < (1ll << 28), "sod_wfm: bad shape");
+  DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_wfm: workspace must be 256-byte aligned");
+  return launch_sod_wfm(pred, gt, ws, out, B, Sized{sizes, Hmax, Wmax}, (cudaStream_t)stream);
 }
 
 }  // extern "C"

@@ -1,6 +1,8 @@
 // Memory/latency-bound pieces of the texture diffuser: surface normals (a1), the fused
 // diffusion front (a3..a6), the stand-alone MessagePassing operator fwd/bwd (a6), and the
 // small NCHW helpers that make every nn.Module of the path callable on its own.
+#include <math_constants.h>
+
 #include "common.cuh"
 
 namespace dgtd {
@@ -154,6 +156,16 @@ __global__ void conv1x1_nchw_kernel(const float* __restrict__ x, const float* __
   out[((int64_t)b * Cout + co) * HW + p] = acc;
 }
 
+// bilinear sample (align_corners=False) of the (h, w) plane p at output pixel (oy, ox) of an (oh, ow) resize
+__device__ __forceinline__ float bilinear_at(const float* __restrict__ p, int h, int w, int oh, int ow, int oy, int ox) {
+  int y0, y1, x0, x1;
+  float ly, lx;
+  bilinear_src(oy, (float)h / oh, h, y0, y1, ly);
+  bilinear_src(ox, (float)w / ow, w, x0, x1, lx);
+  return (1.f - ly) * ((1.f - lx) * p[(int64_t)y0 * w + x0] + lx * p[(int64_t)y0 * w + x1]) +
+         ly * ((1.f - lx) * p[(int64_t)y1 * w + x0] + lx * p[(int64_t)y1 * w + x1]);
+}
+
 __global__ void resize_nchw_kernel(const float* __restrict__ x, float* __restrict__ out, int h, int w,
                                    int oh, int ow, int bilinear) {
   int plane = blockIdx.z;
@@ -162,18 +174,33 @@ __global__ void resize_nchw_kernel(const float* __restrict__ x, float* __restric
   const float* p = x + (int64_t)plane * h * w;
   float v;
   if (bilinear) {
-    int y0, y1, x0, x1;
-    float ly, lx;
-    bilinear_src(oy, (float)h / oh, h, y0, y1, ly);
-    bilinear_src(ox, (float)w / ow, w, x0, x1, lx);
-    v = (1.f - ly) * ((1.f - lx) * p[(int64_t)y0 * w + x0] + lx * p[(int64_t)y0 * w + x1]) +
-        ly * ((1.f - lx) * p[(int64_t)y1 * w + x0] + lx * p[(int64_t)y1 * w + x1]);
+    v = bilinear_at(p, h, w, oh, ow, oy, ox);
   } else {
     int sy = min((int)floorf(oy * ((float)h / oh)), h - 1);
     int sx = min((int)floorf(ox * ((float)w / ow)), w - 1);
     v = p[(int64_t)sy * w + sx];
   }
   out[((int64_t)plane * oh + oy) * ow + ox] = v;
+}
+
+// Predict head for images of different sizes: plane b (h, w) -> sigmoid of its bilinear resize to sizes[b] = (H_b, W_b)
+// in the top-left of an (Hmax, Wmax) plane, 0 in the rest.  Per image the same arithmetic as resize_nchw_kernel then
+// sigmoid_kernel; a plane already at (H_b, W_b) is copied, as `Hitnet.predict_logits` skips that resize.  A size
+// outside [2, Hmax] x [2, Wmax] fills the whole plane with NaN.
+__global__ void resize_sigmoid_sized_kernel(const float* __restrict__ x, float* __restrict__ out,
+                                            const int* __restrict__ sizes, int h, int w, int Hmax, int Wmax) {
+  const int b = blockIdx.z;
+  const int ox = blockIdx.x * blockDim.x + threadIdx.x, oy = blockIdx.y * blockDim.y + threadIdx.y;
+  if (ox >= Wmax || oy >= Hmax) return;
+  const int oh = sizes[2 * b], ow = sizes[2 * b + 1];
+  float v = 0.f;
+  if (!(oh >= 2 && oh <= Hmax && ow >= 2 && ow <= Wmax)) {
+    v = CUDART_NAN_F;
+  } else if (oy < oh && ox < ow) {
+    const float* p = x + (int64_t)b * h * w;
+    v = sigmoidf_acc((oh == h && ow == w) ? p[(int64_t)oy * w + ox] : bilinear_at(p, h, w, oh, ow, oy, ox));
+  }
+  out[((int64_t)b * Hmax + oy) * Wmax + ox] = v;
 }
 
 // Generic LayerNorm over the middle dim of (outer, C, inner); one warp per (outer, inner) row,
@@ -518,6 +545,16 @@ int dgtd_resize_nchw_fwd(const float* x, float* out, int planes, int h, int w, i
   dim3 block(32, 8), grid(cdiv(ow, 32), cdiv(oh, 8), planes);
   resize_nchw_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(x, out, h, w, oh, ow, bilinear);
   DGTD_LAUNCH_CHECK("resize_nchw");
+  return 0;
+}
+
+int dgtd_resize_sigmoid_sized_fwd(const float* x, float* out, const int32_t* sizes, int B, int h, int w, int Hmax,
+                                  int Wmax, dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(x && out && sizes && B > 0 && h > 0 && w > 0 && Hmax > 1 && Wmax > 1, "resize_sigmoid_sized: bad args");
+  DGTD_CHECK_ARG(B <= 65535, "resize_sigmoid_sized: too many planes");
+  dim3 block(32, 8), grid(cdiv(Wmax, 32), cdiv(Hmax, 8), B);
+  resize_sigmoid_sized_kernel<<<grid, block, 0, (cudaStream_t)stream>>>(x, out, sizes, h, w, Hmax, Wmax);
+  DGTD_LAUNCH_CHECK("resize_sigmoid_sized");
   return 0;
 }
 

@@ -26,6 +26,7 @@ from ..ops.functions import hitnet_func as HF
 from ..ops.functions import hitnet_train_func as HT
 from ..ops.functions import texture_diffusion_func as OP
 from ..ops.capi import BF16
+from ..padded import PaddedBatch
 from .pvt import pvt_v2_b2
 from .texture_diffuser import _mode, _packed, _wants_grad
 
@@ -445,7 +446,12 @@ class cod(nn.Module):
 
     `forward(raw, input, label, depth, mode)`: 'predict' -> (sigmoid(output), label) like cod.py:217 without the
     PNG side effects; 'tensor' -> output logits; 'loss' -> {'loss': loss_p1 + loss_P2 + loss_3} of cod.py:135-146
-    with an autograd graph to every parameter when gradients are enabled (the training step of cod.py:118-146)."""
+    with an autograd graph to every parameter when gradients are enabled (the training step of cod.py:118-146).
+
+    'predict' with `label` a list of maps of different sizes (the public COD test sets keep each mask at its source
+    resolution) predicts the batch once and resizes image b's logits to its own label's size, like cod.py:149 does
+    one image at a time.  It returns (probabilities, labels) as two `PaddedBatch` on the input's device, which the
+    evaluators of twig/metric take as they are.  'tensor' does not take such labels."""
 
     def __init__(self, win_size=None, filter_ratio=None, using_depth=None, using_sam=None, finetune=None,
                  binary_thresh=None, pretrain_sam=None, head=None):
@@ -457,10 +463,19 @@ class cod(nn.Module):
     def forward(self, raw, input, label, depth, mode='loss'):
         if isinstance(input, (tuple, list)):
             input = torch.stack(input, dim=0)
-        if isinstance(label, (tuple, list)):
+        ragged = (mode in ('predict', 'tensor') and isinstance(label, (tuple, list))
+                  and len({tuple(lb.shape[-2:]) for lb in label}) > 1)
+        if isinstance(label, (tuple, list)) and not ragged:
             label = torch.stack(label, dim=0)
         if isinstance(depth, (tuple, list)):
             depth = torch.stack(depth, dim=0)
+        if ragged:
+            if mode == 'tensor':
+                raise NotImplementedError("mode='tensor' takes labels of one size only")
+            with torch.no_grad():
+                labels = PaddedBatch.from_list(label, device=input.device)
+                _, output = self.hitnet.predict_logits(input, depth, None)
+                return HF.resize_sigmoid_sized(output, labels), labels
         if mode in ('predict', 'tensor'):
             with torch.no_grad():
                 size = label.shape[-2:] if label is not None else None

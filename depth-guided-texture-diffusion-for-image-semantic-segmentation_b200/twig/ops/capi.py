@@ -42,6 +42,7 @@ SIGNATURES = {
     "dgtd_conv1x1_nchw_bwd": [_P, _P, _P, _P, _P, _P, _P, _I, _I, _I, _I, _P],
     "dgtd_resize_bilinear_nchw_bwd": [_P, _P, _I, _I, _I, _I, _I, _P],
     "dgtd_resize_nchw_fwd": [_P, _P, _I, _I, _I, _I, _I, _I, _P],
+    "dgtd_resize_sigmoid_sized_fwd": [_P, _P, _P, _I, _I, _I, _I, _I, _P],
     "dgtd_layer_norm_fwd": [_P, _P, _P, _P, _L, _I, _L, _F, _P],
     "dgtd_stem_fwd": [_P, _P, _I, _P, _P, _P, _P, _P, _I, _I, _I, _I, _F, _P],
     "dgtd_ln_patchify_fwd": [_P, _P, _P, _P, _I, _I, _I, _I, _I, _F, _P],
@@ -133,6 +134,8 @@ SIGNATURES = {
     "dgtd_sod_metrics_fwd": [_P, _P, _P, _P, _P, _I, _I, _I, _P],
     "dgtd_sod_wfm_ws_bytes": [_I, _I, _I],
     "dgtd_sod_wfm_fwd": [_P, _P, _P, _P, _I, _I, _I, _P],
+    "dgtd_sod_metrics_sized_fwd": [_P, _P, _P, _P, _P, _P, _I, _I, _I, _P],
+    "dgtd_sod_wfm_sized_fwd": [_P, _P, _P, _P, _P, _I, _I, _I, _P],
 }
 _RESTYPES = {"dgtd_last_error": c_char_p, "dgtd_launch_count": c_int64, "dgtd_sod_metrics_ws_bytes": c_int64,
              "dgtd_sod_wfm_ws_bytes": c_int64,

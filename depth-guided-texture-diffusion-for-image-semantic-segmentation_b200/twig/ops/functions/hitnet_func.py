@@ -10,8 +10,10 @@ import torch
 
 from .. import capi
 from ..capi import call, check_cuda, ptr, stream
+from ...padded import PaddedBatch
 
-__all__ = ["conv_affine", "conv_affine_tc", "conv3_tc", "channel_sums", "channel_gate", "gated_sum", "resize_ld", "copy_channels", "head1", "sigmoid"]
+__all__ = ["conv_affine", "conv_affine_tc", "conv3_tc", "channel_sums", "channel_gate", "gated_sum", "resize_ld", "copy_channels", "head1", "sigmoid",
+           "resize_sigmoid_sized"]
 
 
 def _on_cuda(*tensors: Optional[torch.Tensor]) -> None:
@@ -179,4 +181,17 @@ def sigmoid(x: torch.Tensor) -> torch.Tensor:
     x = x.contiguous()
     out = torch.empty_like(x)
     call("dgtd_sigmoid_fwd", ptr(x), ptr(out), x.numel(), stream())
+    return out
+
+
+def resize_sigmoid_sized(x: torch.Tensor, like: PaddedBatch) -> PaddedBatch:
+    """(B,1,h,w) logits -> a PaddedBatch with `like`'s sizes holding per image `sigmoid(resize_nchw(x[b], (H_b,
+    W_b)))`, bit for bit (0 in the padding)."""
+    check_cuda(x)
+    B, C, h, w = x.shape
+    assert C == 1 and B == len(like) and x.dtype == torch.float32, (tuple(x.shape), x.dtype, len(like))
+    out = like.empty_like()
+    _, _, Hmax, Wmax = out.data.shape
+    call("dgtd_resize_sigmoid_sized_fwd", ptr(x), ptr(out.data), ptr(out.device_sizes()), B, h, w, Hmax, Wmax,
+         stream())
     return out

@@ -136,6 +136,12 @@ int dgtd_resize_bilinear_nchw_bwd(const float* grad_out, float* grad_x, int plan
  * nearest (cod.py:1295). */
 int dgtd_resize_nchw_fwd(const float* x, float* out, int planes, int h, int w, int oh, int ow,
                          int bilinear, dgtd_stream_t stream);
+/* predict head for ground truths of different sizes: x (B,1,h,w) logits -> out (B,1,Hmax,Wmax), where image b is
+ * sigmoid(bilinear resize of plane b to sizes[b] = (H_b, W_b)) in the top-left H_b x W_b and 0 elsewhere; bit for bit
+ * dgtd_resize_nchw_fwd to (H_b, W_b) then dgtd_sigmoid_fwd (a plane already at (H_b, W_b) is copied).  sizes: device
+ * int32 (B, 2), 2 <= H_b <= Hmax and 2 <= W_b <= Wmax; an image whose size breaks that is all NaN. */
+int dgtd_resize_sigmoid_sized_fwd(const float* x, float* out, const int32_t* sizes, int B, int h, int w, int Hmax,
+                                  int Wmax, dgtd_stream_t stream);
 /* custom LayerNorm, cod.py:1041-1049: x viewed as (outer, C, inner); channels_last: inner=1 */
 int dgtd_layer_norm_fwd(const float* x, const float* w, const float* b, float* out, int64_t outer,
                         int C, int64_t inner, float eps, dgtd_stream_t stream);
@@ -501,6 +507,15 @@ int dgtd_sod_metrics_fwd(const float* pred, const float* gt, void* ws, double* o
 int64_t dgtd_sod_wfm_ws_bytes(int B, int H, int W);
 int dgtd_sod_wfm_fwd(const float* pred, const float* gt, void* ws, double* out, int B, int H, int W,
                      dgtd_stream_t stream);
+/* The same two evaluations for images of different sizes in one padded batch: pred, gt (B,1,Hmax,Wmax), image b in
+ * the top-left sizes[b] = (H_b, W_b) of its plane; the rest of the plane is never read.  sizes: device int32 (B, 2)
+ * with 2 <= H_b <= Hmax and 2 <= W_b <= Wmax; an image whose size breaks that reads nothing and gets NaN results.
+ * Image b's out, curves and F^w are bit-identical to dgtd_sod_metrics_fwd / dgtd_sod_wfm_fwd on its contiguous
+ * H_b x W_b crop alone.  ws: dgtd_sod_metrics_ws_bytes(B, Hmax, Wmax) / dgtd_sod_wfm_ws_bytes(B, Hmax, Wmax). */
+int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out,
+                               double* curves, int B, int Hmax, int Wmax, dgtd_stream_t stream);
+int dgtd_sod_wfm_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out, int B,
+                           int Hmax, int Wmax, dgtd_stream_t stream);
 
 /* ---- optimizer step of the training configuration (config/sod.yml:56-76; torch.optim.AdamW semantics) ----------
  * One launch over flat fp32 buffers p, g, m, v (the hot path's gradients already live in one flat buffer,
