@@ -517,6 +517,22 @@ int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t
 int dgtd_sod_wfm_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out, int B,
                            int Hmax, int Wmax, dgtd_stream_t stream);
 
+/* ---- dataset preprocessing of decoded RGB-D images (SURVEY §2 row 11: twig/dataset/*.py) --------------------------
+ * Bit-identical to the datasets' host transforms of each image at its own size: PIL 12.2 bilinear Resize to
+ * (out_h, out_w), ToTensor and Normalize(mean, std) for the RGB; convert('L') (for a 3-channel depth), Resize and
+ * ToTensor for the depth.  packed: device uint8, 8-byte aligned, of packed_bytes bytes.  Its head is B descriptors of
+ * 7 int64 = {RGB byte offset, H, W, depth byte offset, H', W', depth channels (1 or 3)}; the offsets point into the
+ * same buffer at the RGB plane (H, W, 3) and the depth plane (H', W', channels), uint8, contiguous.  Every side is
+ * 1..65535, max_h / max_w bound every H, H' / W, W' of the batch.  Outputs: image (B, 3, out_h, out_w) and depth
+ * (B, 1, out_h, out_w) fp32 NCHW.  An image whose descriptor breaks these bounds, or that does not fit ws, gets NaN.
+ * Four launches over the whole batch, integer arithmetic after float64 coefficients, no atomics: an image's output
+ * does not depend on its batch.  ws: 256-byte aligned scratch of dgtd_rgbd_preprocess_ws_bytes(desc, B, out_h,
+ * out_w), where desc is a HOST copy of the descriptor table (-1 when a descriptor is out of range). */
+int64_t dgtd_rgbd_preprocess_ws_bytes(const int64_t* desc, int B, int out_h, int out_w);
+int dgtd_rgbd_preprocess_fwd(const void* packed, int64_t packed_bytes, int B, int max_h, int max_w, int out_h,
+                             int out_w, float mean0, float mean1, float mean2, float std0, float std1, float std2,
+                             void* ws, int64_t ws_bytes, float* image, float* depth, dgtd_stream_t stream);
+
 /* ---- optimizer step of the training configuration (config/sod.yml:56-76; torch.optim.AdamW semantics) ----------
  * One launch over flat fp32 buffers p, g, m, v (the hot path's gradients already live in one flat buffer,
  * twig/graphs.py).  table: nslices entries of dgtd_adamw_slice_bytes() bytes = {int64 off; int32 n (<= 4096);
