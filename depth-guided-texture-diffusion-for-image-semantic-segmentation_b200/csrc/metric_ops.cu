@@ -219,13 +219,14 @@ __device__ double s_object_from_moments(double n, double S1, double S2, double R
   return 2.0 * x / (x * x + 1.0 + sigma + 2.220446049250313e-16);
 }
 
-template <class G>
+// out[b][0] = MAE, out[b][1] = S-measure; OS doubles per image
+template <class G, int OS>
 __global__ void metric_final_kernel(MetricWs m, int nchunks, int B, G geo, double* __restrict__ out) {
   const int b = blockIdx.x * blockDim.x + threadIdx.x;
   if (b >= B) return;
   const Dims d = geo.dims(b);
   const int H = d.h, W = d.w;
-  if (G::sized && H == 0) { out[b * 2 + 0] = out[b * 2 + 1] = CUDART_NAN; return; }
+  if (G::sized && H == 0) { out[b * OS + 0] = out[b * OS + 1] = CUDART_NAN; return; }
   double S[NS2];
   for (int k = 0; k < NS2; ++k) {
     unsigned long long v = 0;
@@ -241,7 +242,7 @@ __global__ void metric_final_kernel(MetricWs m, int nchunks, int B, G geo, doubl
   }
   const double n_fg = Sg, n_bg = n - Sg;
   // MAE.step: mean |pred - gt| = (sum_bg d + sum_fg (R - d)) / (R n)
-  out[b * 2 + 0] = ((Sd - Sdg) + (n_fg * R - Sdg)) / (R * n);
+  out[b * OS + 0] = ((Sd - Sdg) + (n_fg * R - Sdg)) / (R * n);
   double sm;
   if (n_fg == 0.0) {
     sm = 1.0 - Sd / (R * n);
@@ -269,14 +270,22 @@ __global__ void metric_final_kernel(MetricWs m, int nchunks, int B, G geo, doubl
       sm = sm > 0.0 ? sm : 0.0;
     }
   }
-  out[b * 2 + 1] = sm;
+  out[b * OS + 1] = sm;
+}
+
+// p(u): the min-max normalised prediction of u8 value u, (u/255 - min/255) / (max/255 - min/255), in the library's
+// IEEE order (explicit round-to-nearest intrinsics: no contraction).  dmin = 0, R = 255 is both the constant-prediction
+// convention of metric_info_kernel (no normalisation) and the full-range case, where (p0 - 0) / (1 - 0) == p0 exactly.
+__device__ __forceinline__ double norm_pred(int u, int dmin, int R) {
+  const double p0 = __ddiv_rn((double)u, 255.0);
+  const double mn = __ddiv_rn((double)dmin, 255.0), mx = __ddiv_rn((double)(dmin + R), 255.0);
+  return (dmin == 0 && R == 255) ? p0 : __ddiv_rn(__dsub_rn(p0, mn), __dsub_rn(mx, mn));
 }
 
 // F- / E-measure (pysodmetrics `Fmeasure.cal_pr`, `Emeasure.cal_em_with_cumsumhistogram`): both are functions of the
 // foreground / background histograms of the min-max normalised prediction re-quantised to uint8.  The library
-// does that re-quantisation in float64 -- (u/255 - min/255) / (max/255 - min/255) * 255, truncated -- and a value
-// that lands on an integer can fall either side of it, so the 256-entry map is evaluated with the same IEEE
-// operations in the same order (explicit round-to-nearest intrinsics: no contraction).
+// does that re-quantisation in float64 -- p(u) * 255, truncated -- and a value that lands on an integer can fall
+// either side of it, so the 256-entry map is evaluated with the same IEEE operations in the same order.
 template <class G>
 __global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, G geo) {
   __shared__ unsigned int hist[512];
@@ -285,11 +294,7 @@ __global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, G geo) {
   const int dmin = m.info[b * 4 + 0], R = m.info[b * 4 + 1];
   {
     const int u = threadIdx.x;
-    const double p0 = __ddiv_rn((double)u, 255.0);
-    const double mn = __ddiv_rn((double)dmin, 255.0), mx = __ddiv_rn((double)(dmin + R), 255.0);
-    // dmin = 0, R = 255 is both the constant-prediction convention of metric_info_kernel (no normalisation) and
-    // the full-range case, where (p0 - 0) / (1 - 0) == p0 exactly
-    const double p = (dmin == 0 && R == 255) ? p0 : __ddiv_rn(__dsub_rn(p0, mn), __dsub_rn(mx, mn));
+    const double p = norm_pred(u, dmin, R);
     const int q = (u >= dmin && u <= dmin + R) ? (int)__dmul_rn(p, 255.0) : 0;
     lut[u] = (unsigned char)q;
     hist[u] = 0u;
@@ -310,15 +315,157 @@ __global__ void __launch_bounds__(256) metric_hist_kernel(MetricWs m, G geo) {
   o[256 + threadIdx.x] = hist[256 + threadIdx.x];
 }
 
-// curves[b][0][i] = changeable F-measure, curves[b][1][i] = E-measure at threshold 255 - i (the library's order)
+// ---- adaptive threshold: numpy's `p.mean()` --------------------------------------------------------------------------
+// pysodmetrics binarises at min(2 * p.mean(), 1), and a threshold one ulp off changes the binary map whenever 2 * mean
+// lands on a prediction level, so the mean is summed in numpy's order: `pairwise_sum` over the flattened image, where a
+// block of n <= 128 elements is a leaf (eight accumulators r[k] += a[i + k] for i = 8, 16, ... < n - n % 8, combined as
+// ((r0 + r1) + (r2 + r3)) + ((r4 + r5) + (r6 + r7)), then the n % 8 rest in order; below 8 elements, in order from 0)
+// and a larger block splits at n / 2 - (n / 2) % 8.  The tree depends on N = H_b W_b only.  A node is addressed by the
+// bits of a path from its subtree's root (1 = right child); a node that stops splitting before the path ends is
+// summed once, by the path whose remaining bits are 0, and its value is kept at that position.  The mean kernel sums
+// one "tile" (a node whose leaves are at most PW_CTA_LEVELS splits down) per CTA, 8 lanes per leaf, and combines its
+// leaves in shared memory; the curves tail combines the tiles.  No atomics: the result depends on N and the pixels
+// only, not on how the tree is cut into tiles.
+constexpr int PW_LEAF = 128;
+constexpr int PW_CTA_LEVELS = 7;     // 2^7 leaf positions per CTA, 4 per group of 8 lanes
+
+__host__ __device__ __forceinline__ int pw_left(int n) { return (n >> 1) & ~7; }
+
+// splits from a node of n elements down to its deepest leaf, counted up to `cap`: the right child is never the smaller
+// one, so the deepest leaf is on the right spine
+__host__ __device__ __forceinline__ int pw_depth(int n, int cap) {
+  int d = 0;
+  for (; n > PW_LEAF && d < cap; ++d) n -= pw_left(n);
+  return d;
+}
+
+__device__ __forceinline__ bool pw_is_leaf(int n) { return n <= PW_LEAF; }
+__device__ __forceinline__ bool pw_is_tile(int n) { return pw_depth(n, PW_CTA_LEVELS + 1) <= PW_CTA_LEVELS; }
+
+struct PwNode { int off, n, level; };
+
+// follow the `levels` high bits of `path` down from a root of n elements, stopping early at a node where stop(n)
+template <class Stop>
+__device__ __forceinline__ PwNode pw_descend(int n, int path, int levels, Stop stop) {
+  int off = 0, l = 0;
+  for (; l < levels && !stop(n); ++l) {
+    const int left = pw_left(n);
+    if ((path >> (levels - 1 - l)) & 1) { off += left; n -= left; } else { n = left; }
+  }
+  return {off, n, l};
+}
+
+// tiles per image: 2^(top levels) for any image of at most n pixels (right child <= ceil(n / 2) + 7)
+static int pw_slots(int64_t n) {
+  int d = 0;
+  for (; n > PW_LEAF; ++d) n = (n + 1) / 2 + 7;
+  return 1 << (d > PW_CTA_LEVELS ? d - PW_CTA_LEVELS : 0);
+}
+
+// msum[b][p] = pairwise sum of tile p of image b (p = the tile's path from the root), read through the u8 prediction
+// and the p(u) table
 template <class G>
-__global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchunks, G geo, double* __restrict__ curves) {
+__global__ void __launch_bounds__(256) metric_mean_kernel(MetricWs m, G geo, double* __restrict__ msum, int slots) {
+  __shared__ double tab[256];
+  __shared__ double val[1 << PW_CTA_LEVELS];
+  const int b = blockIdx.y, p = blockIdx.x;
+  const Dims d = geo.dims(b);
+  const int N = d.h * d.w, W = d.w;
+  const int top = max(0, pw_depth(N, 32) - PW_CTA_LEVELS);
+  if (N == 0 || p >= (1 << top)) return;
+  const PwNode tile = pw_descend(N, p, top, pw_is_tile);
+  if (p & ((1 << (top - tile.level)) - 1)) return;          // the tile is summed by a lower path
+  tab[threadIdx.x] = norm_pred(threadIdx.x, m.info[b * 4 + 0], m.info[b * 4 + 1]);
+  __syncthreads();
+  const unsigned char* pu = m.pu8 + (int64_t)b * geo.H * geo.W;
+  const int k = threadIdx.x & 7;
+  for (int pos = threadIdx.x >> 3; pos < (1 << PW_CTA_LEVELS); pos += 32) {     // warp-uniform trip count
+    const PwNode leaf = pw_descend(tile.n, pos, PW_CTA_LEVELS, pw_is_leaf);
+    const bool mine = (pos & ((1 << (PW_CTA_LEVELS - leaf.level)) - 1)) == 0;
+    const int off = tile.off + leaf.off, n = leaf.n, nfull = n - n % 8;
+    double s = 0.0;
+    if (mine && n >= 8) {
+      s = tab[pu[geo.at(off + k, W)]];
+      for (int i = 8 + k; i < nfull; i += 8) s += tab[pu[geo.at(off + i, W)]];
+    }
+    s += __shfl_xor_sync(0xffffffffu, s, 1);
+    s += __shfl_xor_sync(0xffffffffu, s, 2);
+    s += __shfl_xor_sync(0xffffffffu, s, 4);
+    if (mine && k == 0) {
+      for (int i = nfull; i < n; ++i) s += tab[pu[geo.at(off + i, W)]];     // n < 8: s = 0, then every element
+      val[pos] = s;
+    }
+  }
+  __syncthreads();
+  for (int L = PW_CTA_LEVELS - 1; L >= 0; --L) {
+    for (int q = threadIdx.x; q < (1 << L); q += 256) {
+      const PwNode c = pw_descend(tile.n, q, L, pw_is_leaf);
+      if (c.level == L && !pw_is_leaf(c.n))
+        val[q << (PW_CTA_LEVELS - L)] += val[(2 * q + 1) << (PW_CTA_LEVELS - 1 - L)];
+    }
+    __syncthreads();
+  }
+  if (threadIdx.x == 0) msum[(int64_t)b * slots + p] = val[0];
+}
+
+// Emeasure.cal_em_with_cumsumhistogram at one threshold (and cal_em_with_threshold: the same arithmetic and order)
+__device__ __forceinline__ double emeasure(double fg_fg, double fg_bg, double gt_fg, double size) {
+  const double eps = 2.220446049250313e-16;
+  const double pred_fg = fg_fg + fg_bg, pred_bg = size - pred_fg;
+  double total;
+  if (gt_fg == 0.0) {
+    total = pred_bg;
+  } else if (gt_fg == size) {
+    total = pred_fg;
+  } else {
+    const double bg_fg = gt_fg - fg_fg, bg_bg = pred_bg - bg_fg;
+    const double mp = pred_fg / size, mg = gt_fg / size;
+    const double a[2] = {1.0 - mp, 0.0 - mp}, c[2] = {1.0 - mg, 0.0 - mg};
+    const double numel[4] = {fg_fg, fg_bg, bg_fg, bg_bg};
+    total = 0.0;
+#pragma unroll
+    for (int i = 0; i < 4; ++i) {
+      const double x = a[i >> 1], y = c[i & 1];
+      const double align = 2.0 * (x * y) / (x * x + y * y + eps);
+      total += (align + 1.0) * (align + 1.0) / 4.0 * numel[i];
+    }
+  }
+  return total / (size - 1.0 + eps);
+}
+
+// curves[b][0][i] = changeable F-measure, curves[b][1][i] = E-measure at threshold 255 - i (the library's order).
+// FULL: also curves[b][2][i] = precision, curves[b][3][i] = recall, and vals[b][2] = adaptive F-measure, vals[b][3] =
+// adaptive E-measure from the tiles' sums msum[b][.] of metric_mean_kernel (combined here, in place).
+template <class G, bool FULL>
+__global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchunks, G geo, double* __restrict__ curves,
+                                                            double* msum, int slots, double* __restrict__ vals) {
+  constexpr int NC = FULL ? 4 : 2;
   __shared__ double cf[256], cb[256];
+  __shared__ int ustar;
   const int b = blockIdx.x, t = threadIdx.x;
   const Dims d = geo.dims(b);
   if (G::sized && d.h == 0) {
-    curves[((int64_t)b * 2 + 0) * 256 + t] = curves[((int64_t)b * 2 + 1) * 256 + t] = CUDART_NAN;
+#pragma unroll
+    for (int k = 0; k < NC; ++k) curves[((int64_t)b * NC + k) * 256 + t] = CUDART_NAN;
+    if (FULL && t == 0) vals[b * 4 + 2] = vals[b * 4 + 3] = CUDART_NAN;
     return;
+  }
+  if (FULL) {
+    // the levels above the tiles, bottom up, then p(u) >= min(2 * mean, 1) for u >= u* only (p is increasing)
+    const int N = d.h * d.w, top = max(0, pw_depth(N, 32) - PW_CTA_LEVELS);
+    double* ms = msum + (int64_t)b * slots;
+    for (int L = top - 1; L >= 0; --L) {
+      for (int q = t; q < (1 << L); q += 256) {
+        const PwNode c = pw_descend(N, q, L, pw_is_tile);
+        if (c.level == L && !pw_is_tile(c.n)) ms[q << (top - L)] += ms[(2 * q + 1) << (top - 1 - L)];
+      }
+      __syncthreads();
+    }
+    const double thr = fmin(__dmul_rn(2.0, __ddiv_rn(ms[0], (double)N)), 1.0);
+    const int dmin = m.info[b * 4 + 0], R = m.info[b * 4 + 1];
+    if (t == 0) ustar = 256;
+    __syncthreads();
+    if (t >= dmin && t <= dmin + R && norm_pred(t, dmin, R) >= thr) atomicMin(&ustar, t);
   }
   unsigned long long f = 0, g = 0;
   for (int c = 0; c < nchunks; ++c) {
@@ -333,7 +480,6 @@ __global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchu
     for (int i = 1; i < 256; ++i) { cf[i] += cf[i - 1]; cb[i] += cb[i - 1]; }
   }
   __syncthreads();
-  const double eps = 2.220446049250313e-16;
   const double size = (double)d.h * (double)d.w, gt_fg = cf[255];
   const double fg_fg = cf[t], fg_bg = cb[t];
   // Fmeasure.cal_pr, beta^2 = 0.3
@@ -344,30 +490,30 @@ __global__ void __launch_bounds__(256) metric_curves_kernel(MetricWs m, int nchu
     const double prec = fg_fg / ps, rec = fg_fg / T;
     const double num = 1.3 * prec * rec;
     const double den = num == 0.0 ? 1.0 : 0.3 * prec + rec;
-    curves[((int64_t)b * 2 + 0) * 256 + t] = num / den;
-  }
-  // Emeasure.cal_em_with_cumsumhistogram
-  {
-    const double pred_fg = fg_fg + fg_bg, pred_bg = size - pred_fg;
-    double total;
-    if (gt_fg == 0.0) {
-      total = pred_bg;
-    } else if (gt_fg == size) {
-      total = pred_fg;
-    } else {
-      const double bg_fg = gt_fg - fg_fg, bg_bg = pred_bg - bg_fg;
-      const double mp = pred_fg / size, mg = gt_fg / size;
-      const double a[2] = {1.0 - mp, 0.0 - mp}, c[2] = {1.0 - mg, 0.0 - mg};
-      const double numel[4] = {fg_fg, fg_bg, bg_fg, bg_bg};
-      total = 0.0;
-#pragma unroll
-      for (int i = 0; i < 4; ++i) {
-        const double x = a[i >> 1], y = c[i & 1];
-        const double align = 2.0 * (x * y) / (x * x + y * y + eps);
-        total += (align + 1.0) * (align + 1.0) / 4.0 * numel[i];
-      }
+    curves[((int64_t)b * NC + 0) * 256 + t] = num / den;
+    if (FULL) {
+      curves[((int64_t)b * NC + 2) * 256 + t] = prec;
+      curves[((int64_t)b * NC + 3) * 256 + t] = rec;
     }
-    curves[((int64_t)b * 2 + 1) * 256 + t] = total / (size - 1.0 + eps);
+  }
+  curves[((int64_t)b * NC + 1) * 256 + t] = emeasure(fg_fg, fg_bg, gt_fg, size);
+  if (FULL && t == 0) {
+    // the pixels with p >= threshold are those with lut >= lut[u*]: entry 255 - lut[u*] of the cumulative counts
+    const int dmin = m.info[b * 4 + 0], R = m.info[b * 4 + 1], u = ustar;
+    double i_fg = 0.0, i_bg = 0.0;
+    if (u < 256) {
+      const int k = 255 - (int)__dmul_rn(norm_pred(u, dmin, R), 255.0);
+      i_fg = cf[k];
+      i_bg = cb[k];
+    }
+    // Fmeasure.cal_adaptive_fm: its own formula, not the curve's
+    double fm = 0.0;
+    if (i_fg != 0.0) {
+      const double pre = __ddiv_rn(i_fg, __dadd_rn(i_fg, i_bg)), rec = __ddiv_rn(i_fg, gt_fg);
+      fm = __ddiv_rn(__dmul_rn(__dmul_rn(1.3, pre), rec), __dadd_rn(__dmul_rn(0.3, pre), rec));
+    }
+    vals[b * 4 + 2] = fm;
+    vals[b * 4 + 3] = emeasure(i_fg, i_bg, gt_fg, size);
   }
 }
 
@@ -418,13 +564,10 @@ static MetricWs carve_wfm(void* ws, int B, int H, int W, WfmWs* w, size_t* total
   return m;
 }
 
-// tab[b][g][u] = |p(u) - g| with p = (u/255 - min/255) / (max/255 - min/255) in the library's IEEE order
+// tab[b][g][u] = |p(u) - g|
 __global__ void __launch_bounds__(256) wfm_table_kernel(MetricWs m, WfmWs w) {
   const int b = blockIdx.x, u = threadIdx.x;
-  const int dmin = m.info[b * 4 + 0], R = m.info[b * 4 + 1];
-  const double p0 = __ddiv_rn((double)u, 255.0);
-  const double mn = __ddiv_rn((double)dmin, 255.0), mx = __ddiv_rn((double)(dmin + R), 255.0);
-  const double p = (dmin == 0 && R == 255) ? p0 : __ddiv_rn(__dsub_rn(p0, mn), __dsub_rn(mx, mn));
+  const double p = norm_pred(u, m.info[b * 4 + 0], m.info[b * 4 + 1]);
   w.tab[b * 512 + u] = fabs(p);
   w.tab[b * 512 + 256 + u] = fabs(__dsub_rn(p, 1.0));
 }
@@ -602,7 +745,16 @@ __global__ void wfm_final_kernel(MetricWs m, WfmWs w, int nchunks, int ntiles, i
   out[b] = 2.0 * R * P / (R + P + eps);
 }
 
-template <class G>
+// The full table's workspace: carve()'s, then the tiles' sums of the mean pass
+static size_t carve_full(int B, int H, int W, int* slots) {
+  size_t off = 0;
+  carve(nullptr, B, H, W, &off);
+  *slots = pw_slots((int64_t)H * W);
+  return off;
+}
+
+// FULL: out (B, 4) = MAE, S, adaptive F, adaptive E and curves (B, 4, 256) = F, E, precision, recall
+template <bool FULL, class G>
 static int launch_sod_metrics(const float* pred, const float* gt, void* ws, double* out, double* curves, int B, G geo,
                               cudaStream_t s) {
   MetricWs m = carve(ws, B, geo.H, geo.W, nullptr);
@@ -613,12 +765,19 @@ static int launch_sod_metrics(const float* pred, const float* gt, void* ws, doub
   DGTD_LAUNCH_CHECK("sod_metrics(info)");
   metric_moments_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, geo);
   DGTD_LAUNCH_CHECK("sod_metrics(moments)");
-  metric_final_kernel<<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, geo, out);
+  metric_final_kernel<G, FULL ? 4 : 2><<<cdiv(B, 32), 32, 0, s>>>(m, nchunks, B, geo, out);
   DGTD_LAUNCH_CHECK("sod_metrics(final)");
   if (curves) {
     metric_hist_kernel<<<dim3(nchunks, B), 256, 0, s>>>(m, geo);
     DGTD_LAUNCH_CHECK("sod_metrics(hist)");
-    metric_curves_kernel<<<B, 256, 0, s>>>(m, nchunks, geo, curves);
+    double* msum = nullptr;
+    int slots = 0;
+    if (FULL) {
+      msum = (double*)((char*)ws + carve_full(B, geo.H, geo.W, &slots));
+      metric_mean_kernel<<<dim3(slots, B), 256, 0, s>>>(m, geo, msum, slots);
+      DGTD_LAUNCH_CHECK("sod_metrics_full(mean)");
+    }
+    metric_curves_kernel<G, FULL><<<B, 256, 0, s>>>(m, nchunks, geo, curves, msum, slots, out);
     DGTD_LAUNCH_CHECK("sod_metrics(curves)");
   }
   return 0;
@@ -664,7 +823,7 @@ int dgtd_sod_metrics_fwd(const float* pred, const float* gt, void* ws, double* o
   DGTD_CHECK_ARG(pred && gt && ws && out, "sod_metrics: null pointer");
   DGTD_CHECK_ARG(B > 0 && H > 1 && W > 1 && (int64_t)H * W < (1ll << 28), "sod_metrics: bad shape");
   DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics: workspace must be 256-byte aligned");
-  return launch_sod_metrics(pred, gt, ws, out, curves, B, Dense{H, W}, (cudaStream_t)stream);
+  return launch_sod_metrics<false>(pred, gt, ws, out, curves, B, Dense{H, W}, (cudaStream_t)stream);
 }
 
 int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out,
@@ -672,7 +831,30 @@ int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t
   DGTD_CHECK_ARG(pred && gt && sizes && ws && out, "sod_metrics: null pointer");
   DGTD_CHECK_ARG(B > 0 && Hmax > 1 && Wmax > 1 && (int64_t)Hmax * Wmax < (1ll << 28), "sod_metrics: bad shape");
   DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics: workspace must be 256-byte aligned");
-  return launch_sod_metrics(pred, gt, ws, out, curves, B, Sized{sizes, Hmax, Wmax}, (cudaStream_t)stream);
+  return launch_sod_metrics<false>(pred, gt, ws, out, curves, B, Sized{sizes, Hmax, Wmax}, (cudaStream_t)stream);
+}
+
+int64_t dgtd_sod_metrics_full_ws_bytes(int B, int H, int W) {
+  if (B <= 0 || H <= 0 || W <= 0) return 0;
+  int slots = 0;
+  const size_t off = carve_full(B, H, W, &slots);
+  return (int64_t)align256(off + (size_t)B * slots * sizeof(double));
+}
+
+int dgtd_sod_metrics_full_fwd(const float* pred, const float* gt, void* ws, double* vals, double* curves, int B, int H,
+                              int W, dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(pred && gt && ws && vals && curves, "sod_metrics_full: null pointer");
+  DGTD_CHECK_ARG(B > 0 && H > 1 && W > 1 && (int64_t)H * W < (1ll << 28), "sod_metrics_full: bad shape");
+  DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics_full: workspace must be 256-byte aligned");
+  return launch_sod_metrics<true>(pred, gt, ws, vals, curves, B, Dense{H, W}, (cudaStream_t)stream);
+}
+
+int dgtd_sod_metrics_full_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* vals,
+                                    double* curves, int B, int Hmax, int Wmax, dgtd_stream_t stream) {
+  DGTD_CHECK_ARG(pred && gt && sizes && ws && vals && curves, "sod_metrics_full: null pointer");
+  DGTD_CHECK_ARG(B > 0 && Hmax > 1 && Wmax > 1 && (int64_t)Hmax * Wmax < (1ll << 28), "sod_metrics_full: bad shape");
+  DGTD_CHECK_ARG(((uintptr_t)ws & 255) == 0, "sod_metrics_full: workspace must be 256-byte aligned");
+  return launch_sod_metrics<true>(pred, gt, ws, vals, curves, B, Sized{sizes, Hmax, Wmax}, (cudaStream_t)stream);
 }
 
 int64_t dgtd_sod_wfm_ws_bytes(int B, int H, int W) {

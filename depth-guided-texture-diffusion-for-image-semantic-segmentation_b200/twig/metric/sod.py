@@ -8,6 +8,10 @@ back.  The wrappers keep the reference's protocol, including its quirk that ever
 RUNNING mean over all images seen so far and `compute_metrics` averages those records (Smeasure.py:30-36).
 mmengine's `BaseMetric` (collection across ranks) is runner plumbing and out of scope (SURVEY 8).
 
+`sod_metrics_full` and `SODEvaluator` give the whole table that COD papers report (pysodmetrics' `get_results()`:
+adaptive, mean and max F- and E-measure, precision and recall curves, next to S, MAE and F^w) from one pass per batch,
+without a host synchronisation.
+
 Every function and evaluator also takes ground truths of different sizes, as pysodmetrics scores each prediction at
 its own ground truth's resolution: a pair of `PaddedBatch` or a pair of lists of per-image maps.  One call then
 scores the whole batch, and image b's values are bit-identical to a call on its H_b x W_b maps alone.
@@ -22,7 +26,8 @@ from ..ops import capi
 from ..ops.capi import call, check_cuda, ptr, stream
 from ..padded import PaddedBatch
 
-__all__ = ["sod_metrics", "weighted_fmeasure", "MAE", "Smeasure", "Fmeasure", "Emeasure", "WeightedFmeasure"]
+__all__ = ["sod_metrics", "sod_metrics_full", "weighted_fmeasure", "MAE", "Smeasure", "Fmeasure", "Emeasure",
+           "WeightedFmeasure", "SODEvaluator"]
 
 Maps = Union[torch.Tensor, PaddedBatch, Sequence[torch.Tensor]]
 
@@ -65,6 +70,24 @@ def sod_metrics(pred: Maps, gt: Maps, curves: bool = False):
         call("dgtd_sod_metrics_sized_fwd", ptr(pred), ptr(gt), ptr(sizes), ptr(ws), ptr(out), ptr(cur), B, H, W,
              stream())
     return (out, cur) if curves else out
+
+
+def sod_metrics_full(pred: Maps, gt: Maps) -> Tuple[torch.Tensor, torch.Tensor]:
+    """pred, gt as for `sod_metrics` -> (vals, curves) float64: vals (B, 4) = per-image MAE, S-measure, adaptive
+    F-measure and adaptive E-measure (pysodmetrics `cal_adaptive_fm` / `cal_adaptive_em`: the prediction binarised at
+    min(2 * mean, 1)); curves (B, 4, 256) = changeable F-measure, E-measure, precision and recall (entry i = threshold
+    255 - i).  MAE, S and the F / E curves are bit-identical to `sod_metrics(pred, gt, curves=True)`."""
+    pred, gt, sizes = _batch(pred, gt)
+    B, _, H, W = pred.shape
+    ws = torch.empty(int(capi.load().dgtd_sod_metrics_full_ws_bytes(B, H, W)), device=pred.device, dtype=torch.uint8)
+    vals = torch.empty(B, 4, device=pred.device, dtype=torch.float64)
+    cur = torch.empty(B, 4, 256, device=pred.device, dtype=torch.float64)
+    if sizes is None:
+        call("dgtd_sod_metrics_full_fwd", ptr(pred), ptr(gt), ptr(ws), ptr(vals), ptr(cur), B, H, W, stream())
+    else:
+        call("dgtd_sod_metrics_full_sized_fwd", ptr(pred), ptr(gt), ptr(sizes), ptr(ws), ptr(vals), ptr(cur), B, H, W,
+             stream())
+    return vals, cur
 
 
 def weighted_fmeasure(pred: Maps, gt: Maps) -> torch.Tensor:
@@ -173,3 +196,46 @@ class Smeasure(_Running):
 class WeightedFmeasure(_Running):
     """twig/metric/WeightedFmeasure.py (commented out in the reference): pysodmetrics `WeightedFmeasure`."""
     _per_image, _key, _name = staticmethod(weighted_fmeasure), 'wfm', 'WeightedFmeasure'
+
+
+class SODEvaluator:
+    """The whole COD table in one evaluator: per batch one `sod_metrics_full` and one `weighted_fmeasure` call, with
+    the sums kept on the device (no host synchronisation until `evaluate`).
+
+    It aggregates like pysodmetrics' `get_results()`: per-image values (S, F^w, MAE, adaptive E and F) are averaged
+    over every image seen, and the F / E / precision / recall curves are averaged over images before the max or the
+    mean over thresholds is taken.  It does NOT follow the reference wrappers' protocol (MAE, Smeasure, Fmeasure,
+    Emeasure above), which record a running mean per batch and average those records: with batches of unequal
+    weight that protocol gives other numbers.  `evaluate()` returns Smeasure, wFmeasure, MAE, adpEm, meanEm, maxEm,
+    adpFm, meanFm and maxFm as floats, and the mean curves `fm_curve`, `em_curve`, `precision` and `recall` as
+    (256,) float64 numpy arrays (entry i = threshold 255 - i), e.g. for PR plots."""
+    default_prefix = 'COD'
+
+    def __init__(self, collect_device: str = 'cpu', prefix: Optional[str] = None, data_range: Optional[float] = 1.0):
+        self.collect_device = collect_device
+        self.prefix = prefix or self.default_prefix
+        self._vals: Optional[torch.Tensor] = None      # sums over images: MAE, S, adaptive F, adaptive E, F^w
+        self._curves: Optional[torch.Tensor] = None    # sums over images of the four curves
+        self._count = 0
+
+    def process(self, data_batch, data_samples: Tuple[Maps, Maps]) -> None:
+        # a list is packed once and its sizes uploaded once for both calls
+        pred, gt = (x if isinstance(x, PaddedBatch) else _detached(x) if isinstance(x, torch.Tensor)
+                    else PaddedBatch.from_list(x) for x in data_samples)
+        vals, cur = sod_metrics_full(pred, gt)
+        wfm = weighted_fmeasure(pred, gt)
+        v = torch.cat([vals.sum(0), wfm.sum(0, keepdim=True)])
+        c = cur.sum(0)
+        self._vals = v if self._vals is None else self._vals + v
+        self._curves = c if self._curves is None else self._curves + c
+        self._count += vals.shape[0]
+
+    def evaluate(self) -> dict:
+        if self._count == 0:
+            raise ValueError("SODEvaluator.evaluate: no image has been processed")
+        v = (self._vals / self._count).cpu().numpy()
+        fm, em, p, r = (self._curves / self._count).cpu().numpy()
+        return {"Smeasure": float(v[1]), "wFmeasure": float(v[4]), "MAE": float(v[0]),
+                "adpEm": float(v[3]), "meanEm": float(em.mean()), "maxEm": float(em.max()),
+                "adpFm": float(v[2]), "meanFm": float(fm.mean()), "maxFm": float(fm.max()),
+                "fm_curve": fm, "em_curve": em, "precision": p, "recall": r}

@@ -516,6 +516,21 @@ int dgtd_sod_metrics_sized_fwd(const float* pred, const float* gt, const int32_t
                                double* curves, int B, int Hmax, int Wmax, dgtd_stream_t stream);
 int dgtd_sod_wfm_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* out, int B,
                            int Hmax, int Wmax, dgtd_stream_t stream);
+/* The whole table of pysodmetrics' `Fmeasure` / `Emeasure` / `MAE` / `Smeasure` per image in one pass: same inputs as
+ * dgtd_sod_metrics_fwd; vals (B, 4) float64 = MAE, S-measure, adaptive F-measure, adaptive E-measure; curves
+ * (B, 4, 256) float64 = changeable F-measure, E-measure, precision, recall (entry i = threshold 255 - i).  MAE, S and
+ * the F / E curves are bit-identical to dgtd_sod_metrics_fwd.  The adaptive threshold is min(2 mean(p), 1) with the
+ * mean summed in numpy's pairwise order, so the binary map is the library's bit for bit; adaptive F = 1.3 P R /
+ * (0.3 P + R) of that map (0 when it misses the ground truth), adaptive E the E-measure of that map.  No atomics on
+ * floating point: bit-stable, independent of batch composition.  H > 1, W > 1, H * W < 2^28.  ws: 256-byte aligned
+ * scratch of dgtd_sod_metrics_full_ws_bytes(B, H, W).  The sized form takes the padded batch and device sizes of
+ * dgtd_sod_metrics_sized_fwd, with the same rules (bit-identical to the dense call on each crop, NaN for a size out
+ * of range) and ws of dgtd_sod_metrics_full_ws_bytes(B, Hmax, Wmax). */
+int64_t dgtd_sod_metrics_full_ws_bytes(int B, int H, int W);
+int dgtd_sod_metrics_full_fwd(const float* pred, const float* gt, void* ws, double* vals, double* curves, int B, int H,
+                              int W, dgtd_stream_t stream);
+int dgtd_sod_metrics_full_sized_fwd(const float* pred, const float* gt, const int32_t* sizes, void* ws, double* vals,
+                                    double* curves, int B, int Hmax, int Wmax, dgtd_stream_t stream);
 
 /* ---- dataset preprocessing of decoded RGB-D images (SURVEY §2 row 11: twig/dataset/*.py) --------------------------
  * Bit-identical to the datasets' host transforms of each image at its own size: PIL 12.2 bilinear Resize to
